@@ -2,6 +2,7 @@
 """Benchmark of the LDMSeg sampler hot path (BASELINE.json metric: panoptic frames/sec, DDIM-50, 384x1248 KITTI).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME[,NAME...]]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -195,13 +196,9 @@ def run_reference(args):
     n_frames = cfg.get("clip_frames") or cfg["frames_per_gpu"] * world
     ref = CpuReference(args.ddim_steps, cfg["frame"])
     t_tail = ref.tail()
-    budget_s, t_start, times = 240.0, time.perf_counter(), []
-    for i in range(args.warmup + args.steps):
-        dt = ref.unet_step()
-        if i >= args.warmup or time.perf_counter() - t_start > budget_s:
-            times.append(dt)
-        if time.perf_counter() - t_start > budget_s:  # keep the whole arm within a few minutes
-            break
+    for _ in range(args.warmup):
+        ref.unet_step()
+    times = [ref.unet_step() for _ in range(args.steps)]
     t_unet = float(np.mean(times))
     fps = 1.0 / (args.ddim_steps * t_unet + t_tail)
     cd = config_dict(name, cfg, n_frames, args.ddim_steps, world)
@@ -222,6 +219,42 @@ def frame_digests(ids):
     """[n, H, W] int32 device tensor -> list of per-frame sha256 prefixes."""
     a = np.ascontiguousarray(ids.detach().to("cpu", torch.int32).numpy())
     return [hashlib.sha256(a[i].tobytes()).hexdigest()[:12] for i in range(a.shape[0])]
+
+
+DUMP_BYTES = 64 * 10 ** 6   # --dump-outputs writes at most this much, split evenly over the configs of the run
+PQ_FIELDS = ("pq", "sq", "rq", "tp", "fp", "fn", "iou_sum", "thing_pq", "thing_sq", "thing_rq", "stuff_pq", "stuff_sq",
+             "stuff_rq")
+CLASS_FIELDS = ("pq", "sq", "rq", "tp", "fp", "fn")
+DVPQ_FIELDS = ("iou", "tp", "fn", "fp")
+
+
+def dump_outputs(out_dir, name, wl, res, budget):
+    """What the last timed step returned to its caller, one float array per file out_dir/<config>_<array>.npy:
+      ids            merged panoptic ids (-1 = void) of rank 0's frames, float32 [frames, H, W]; when all frames would
+                     exceed `budget` bytes, a fixed seeded sample of whole frames
+      ids_frames     global index of each frame in `ids`, float64
+      pq             the PQ evaluator's totals in PQ_FIELDS order, float64
+      pq_per_class   one row per class present: class id, then CLASS_FIELDS, float64
+      dvpq_k<k>      DVPQ statistics over windows of k frames, rows DVPQ_FIELDS x 19 classes, float64
+      dvpq_k<k>_pq   pq, pq_things, pq_stuff, number of windows, float64
+    PQ and DVPQ cover the whole clip (all ranks)."""
+    os.makedirs(out_dir, exist_ok=True)
+    frame_bytes = wl.H * wl.W * 4
+    keep = np.arange(wl.n_local)
+    if wl.n_local * frame_bytes > budget:
+        keep = np.sort(np.random.default_rng(0).choice(wl.n_local, max(1, budget // frame_bytes), replace=False))
+    arrays = {
+        "ids": wl.ids_host.numpy()[keep].astype(np.float32),   # ids are below 2^24: exact in float32
+        "ids_frames": (wl.lo + keep).astype(np.float64),
+        "pq": np.array([res[k] for k in PQ_FIELDS], np.float64),
+        "pq_per_class": np.array([[c] + [m[k] for k in CLASS_FIELDS] for c, m in sorted(res["per_class"].items())],
+                                 np.float64).reshape(-1, 1 + len(CLASS_FIELDS)),
+    }
+    for k, v in res["dvpq"].items():
+        arrays[f"dvpq_k{k}"] = np.stack([np.asarray(v[f], np.float64) for f in DVPQ_FIELDS])
+        arrays[f"dvpq_k{k}_pq"] = np.array([v["pq"], v["pq_things"], v["pq_stuff"], v["n_windows"]], np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}_{k}.npy"), a)
 
 
 class Workload:
@@ -335,17 +368,19 @@ def run_config(name, args, env):
         cs = ClockSampler(local) if sample_clocks else None
         if cs:
             cs.start()
-        n0 = L.launch_count()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(steps):
-            res = wl.step(resident)
-        e1.record()
-        torch.cuda.synchronize()
-        if world > 1:
-            dist.barrier()
-        ms = e0.elapsed_time(e1)
-        clocks = cs.stop() if cs else None
+        try:
+            n0 = L.launch_count()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(steps):
+                res = wl.step(resident)
+            e1.record()
+            torch.cuda.synchronize()
+            if world > 1:
+                dist.barrier()
+            ms = e0.elapsed_time(e1)
+        finally:   # the sampler is a child process: never leave it running
+            clocks = cs.stop() if cs else None
         if world > 1:
             t = torch.tensor([ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -359,8 +394,10 @@ def run_config(name, args, env):
     n_batches = len(list(wl.batches()))
     graph_launches = plan.launches_per_forward * T * n_batches * args.steps if plan.graph is not None else 0
     fps = wl.n_frames * args.steps / (ms / 1e3)
-    ms_e2e, _, _, _ = timed(False, 1 if warm else 0, args.steps)      # same number of steps as `value`
+    ms_e2e, res_e2e, _, _ = timed(False, 1 if warm else 0, args.steps)      # same number of steps as `value`
     fps_e2e = wl.n_frames * args.steps / (ms_e2e / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, name, wl, res_e2e, DUMP_BYTES // len(args.config.split(",")))
 
     # digests: identical ids / integer statistics at N = 1 and N > 1 for the same global frames
     digs = frame_digests(wl.cleaned)
@@ -641,7 +678,15 @@ def main():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--ln-fold", action="store_true", help="A/B: LayerNorm folded into the GEMMs around it instead of its own pass (slower, see DESIGN.md)")
     ap.add_argument("--profile-out", default=None, help="write the per-launch CUDA-event profile of one UNet forward")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (panoptic ids, PQ and DVPQ statistics) to "
+                         "DIR/<config>_<array>.npy, at most 64 MB in all; the inputs are seeded, so two builds run with "
+                         "the same arguments can be compared array for array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     for name in args.config.split(","):
         if name not in CONFIGS:
             ap.error(f"unknown config {name!r}")

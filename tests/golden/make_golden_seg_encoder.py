@@ -4,6 +4,10 @@ stores its state_dict, the moments, the posterior's mode / std and ``forward(sam
 Authoring container only (needs /root/reference).
 
     python tests/golden/make_golden_seg_encoder.py     -> tests/golden/seg_encoder_small.npz
+                                                          tests/golden/seg_encoder_small_part2.npz
+
+Random float32 weights do not compress, so the arrays are spread over two files to keep each under 1 MB: the input,
+the outputs, cfg and the encoder's output convolution go to the second one.
 """
 import os
 import sys
@@ -39,9 +43,11 @@ def main():
         post = vae.encode(bits).latent_dist
         out = vae(bits, sample_posterior=False)
     sd = {k: v.numpy() for k, v in vae.state_dict().items()}
-    np.savez_compressed(os.path.join(HERE, "seg_encoder_small.npz"), bits=bits.numpy(), moments=post.parameters.numpy(),
-                        mode=post.mode().numpy(), std=post.std.numpy(), forward=out.sample.numpy(),
-                        cfg=np.array(repr(CFG)), **{"sd." + k: v for k, v in sd.items()})
+    arrays = dict(bits=bits.numpy(), moments=post.parameters.numpy(), mode=post.mode().numpy(), std=post.std.numpy(),
+                  forward=out.sample.numpy(), cfg=np.array(repr(CFG)), **{"sd." + k: v for k, v in sd.items()})
+    part2 = {"bits", "moments", "mode", "std", "forward", "cfg", "sd.encoder.15.weight", "sd.encoder.15.bias"}
+    np.savez_compressed(os.path.join(HERE, "seg_encoder_small.npz"), **{k: v for k, v in arrays.items() if k not in part2})
+    np.savez_compressed(os.path.join(HERE, "seg_encoder_small_part2.npz"), **{k: v for k, v in arrays.items() if k in part2})
     print("wrote seg_encoder_small.npz", post.parameters.shape, out.sample.shape, sorted(k for k in sd if k.startswith("encoder"))[:12])
 
 

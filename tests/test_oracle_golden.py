@@ -144,9 +144,10 @@ def test_seg_encoder_bit_exact_with_reference():
     """oracle.SegEncoderOracle / SegDecoderOracle == the real GeneralVAESeg encoder, posterior and forward()."""
     import ast
     from oracle import ldmseg_oracle as LO
-    z = np.load(os.path.join(G, "seg_encoder_small.npz"))
+    z = {k: f[k] for name in ("seg_encoder_small.npz", "seg_encoder_small_part2.npz")
+         for f in [np.load(os.path.join(G, name))] for k in f.files}
     cfg = ast.literal_eval(str(z["cfg"]))
-    sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")}
+    sd = {k[3:]: torch.from_numpy(v) for k, v in z.items() if k.startswith("sd.")}
     enc = LO.SegEncoderOracle(**cfg).eval()
     enc.load_state_dict({k: v for k, v in sd.items() if k.startswith("encoder.")})
     dec = LO.SegDecoderOracle(**cfg).eval()

@@ -108,10 +108,11 @@ def test_seg_encoder_reference_fixture():
     """encode / posterior / forward of the seg-AE against the real reference (tests/golden/seg_encoder_small.npz)."""
     import ast
     from video_latent_diffusion_panoptic_segmentation_b200.ldmseg.models import GeneralVAESeg
-    z = np.load(os.path.join(G, "seg_encoder_small.npz"))
+    z = {k: f[k] for name in ("seg_encoder_small.npz", "seg_encoder_small_part2.npz")
+         for f in [np.load(os.path.join(G, name))] for k in f.files}
     cfg = ast.literal_eval(str(z["cfg"]))
     vae = GeneralVAESeg(**cfg, device=DEV)
-    vae.load_state_dict({k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd.")})
+    vae.load_state_dict({k[3:]: torch.from_numpy(v) for k, v in z.items() if k.startswith("sd.")})
     bits = torch.from_numpy(z["bits"]).to(DEV)
     post = vae.encode(bits).latent_dist
     assert post.parameters.shape == z["moments"].shape
