@@ -1,6 +1,7 @@
 """Per-kernel parity checks (GPU). Each ``check_*`` returns a dict with error statistics and raises AssertionError
-on failure. The checker is plain PyTorch fp32 math (or numpy/scipy for the integer tail) on the same seeded inputs;
-the thing under test always goes through the C ABI (ops.py -> libldmseg_b200.so).
+on failure. The checker is plain PyTorch fp32 math (or numpy/scipy for the integer tail; fp64 with a bound derived from
+the arithmetic for the attention edge and norm cancellation checks) on the same seeded inputs; the thing under test
+always goes through the C ABI (ops.py -> libldmseg_b200.so).
 
 Used by tests/test_kernels_gpu.py (pytest -m gpu) and by tools/gpu_diag.py (one subprocess per check, so a trapped
 kernel cannot take the other checks down with it).
@@ -61,6 +62,99 @@ def _stats(got, ref, name, atol, rtol):
         res["first_bad"] = idx
         raise AssertionError(f"{name}: {res}")
     return res
+
+
+# ----------------------------------------------------------------------------------------------------------- bound
+# Checks against an fp64 reference with a bound derived from the arithmetic instead of atol + rtol |ref|:
+#     |got - ref| <= r |ref| + a mag
+# mag is the same operation on absolute values (sum_j p_ij |v_j| for attention, |gamma x_hat| + |beta| for the norms):
+# it is the scale of the intermediate values, which is what fp32 accumulation and the rounding of intermediates err
+# against. r covers the rounding of the output; a covers everything before it. The constants have to satisfy two
+# conditions: the kernels stay at or below a quarter of the bound (BOUND_HEADROOM, asserted by the GPU checks), and
+# small, plausible bugs in a reference go above it (tests/test_bound_controls.py, on the CPU).
+U_BF16 = 2.0 ** -8           # unit roundoff of bf16 (8 significant bits): the rounding of a bf16 output
+BOUND_HEADROOM = 0.25
+# attention: the bf16 P perturbs the numerator by up to u mag and, at d = 80 / 160 where the row sum stays fp32 (not the
+# ones row of the same bf16 P), the quotient by up to u |out| <= u mag: one bf16 ulp, seen on the B200 for constant V.
+# MUFU / polynomial ex2 (~1e-4) and fp32 accumulation over <= 7 488 keys are far below u. With the output rounding,
+# a correct kernel errs by up to u |ref| + 2u mag <= 3u mag; a = 11u makes the bound at least four times that.
+A_ATTN = 11 * U_BF16
+# GroupNorm / LayerNorm: GroupNorm takes E[x^2] - mean^2. Its fp32 partial sums are nested sequential sums of a few
+# dozen terms per level (a thread's pixels, the pixel lanes, a group's channels, or a warp tree), and only the fold over
+# CTAs is fp64. Their relative error eps is ~40 * 2^-24 ~ 2^-19 worst case and ~2^-22 for rounding of random sign.
+# The variance carries eps (1 + (mean / spread)^2) / 2 into rstd. For the 64x groups of the cancellation checks, that
+# is ~2^-11 typically; the B200 measures ~2^-13 (worst ratio 0.207 against the 0.2 of the output rounding alone). The
+# worst case, ~2^-8, would reach the bound. LayerNorm is two-pass (~2^-20). The fp32 affine adds ~2^-23. 4u keeps the
+# output rounding under a quarter of the bound, as for attention.
+A_NORM = 4 * U_BF16
+
+
+def bound_ratio(got, ref, mag, r, a):
+    """err / (r |ref| + a mag), elementwise in fp64; NaN / inf in `got` (or an error where the bound is 0) give inf."""
+    ref = ref.double()
+    err = (got.double() - ref).abs()
+    ratio = err / (r * ref.abs() + a * mag.double())
+    return torch.where(torch.isfinite(err) & ((err == 0) | torch.isfinite(ratio)), ratio.nan_to_num(0.0),
+                       torch.full_like(ratio, float("inf")))
+
+
+def _bound_stats(got, ref, mag, name, r, a, limit=BOUND_HEADROOM, where=None):
+    """Raise AssertionError if some element exceeds `limit` x the bound. `where(index)` names a bad element's place in
+    the kernel's work decomposition (tile, warp slice, ...)."""
+    ratio = bound_ratio(got, ref, mag, r, a)
+    worst = ratio.max().item()
+    bad = ratio > limit
+    res = {"name": name, "worst_ratio": worst, "n_bad": int(bad.sum().item()), "n": ratio.numel(),
+           "nan": bool(torch.isnan(got.float()).any().item())}
+    if res["n_bad"]:
+        idx = tuple(bad.nonzero()[0].tolist())
+        res["first_bad"] = idx
+        res["first_bad_got_ref_mag"] = (got[idx].item(), ref[idx].item(), mag[idx].item())
+        if where is not None:
+            res["first_bad_at"] = where(idx)
+        raise AssertionError(f"{name}: {res['n_bad']} of {res['n']} elements above {limit} x bound: {res}")
+    return res
+
+
+def attn_ref(q, k, v, scale, qblock=1024):
+    """softmax(q k^T * scale) v in fp64, the row maximum subtracted, per (image, head) and per query block (no
+    [seq, kv_seq] matrix for all heads at once). q [BH, S, d], k / v [BH, kv_seq, d]: the bf16 values the kernel read.
+    Returns (ref, mag), mag = sum_j p_ij |v_j|."""
+    BH, S, d = q.shape
+    ref = torch.empty((BH, S, d), dtype=torch.float64, device=q.device)
+    mag = torch.empty_like(ref)
+    for b in range(BH):
+        kb, vb = k[b].double(), v[b].double()
+        for i0 in range(0, S, qblock):
+            s = (q[b, i0:i0 + qblock].double() @ kb.t()) * scale
+            p = torch.exp(s - s.max(dim=-1, keepdim=True).values)
+            p /= p.sum(dim=-1, keepdim=True)
+            ref[b, i0:i0 + qblock] = p @ vb
+            mag[b, i0:i0 + qblock] = p @ vb.abs()
+    return ref, mag
+
+
+def norm_ref(x, gamma, beta, eps, groups=None, silu=False):
+    """GroupNorm (groups given; x [B, HW, C], groups of C / groups channels over all pixels) or LayerNorm (x [rows, C])
+    in fp64, two-pass moments. Returns (ref, mag), mag = |gamma x_hat| + |beta| (SiLU: its slope is below 1.1)."""
+    xd = x.double()
+    if groups is None:
+        mean = xd.mean(-1, keepdim=True)
+        var = (xd - mean).pow(2).mean(-1, keepdim=True)
+        xh = (xd - mean) / torch.sqrt(var + eps)
+    else:
+        B, HW, C = xd.shape
+        xg = xd.view(B, HW, groups, C // groups)
+        mean = xg.mean(dim=(1, 3), keepdim=True)
+        var = (xg - mean).pow(2).mean(dim=(1, 3), keepdim=True)
+        xh = ((xg - mean) / torch.sqrt(var + eps)).view(B, HW, C)
+    g, b = gamma.double(), beta.double()
+    y = xh * g + b
+    mag = (xh * g).abs() + b.abs()
+    if silu:
+        y = y * torch.sigmoid(y)
+        mag = 1.1 * mag
+    return y, mag
 
 
 # ----------------------------------------------------------------------------------------------------------- DDIM
@@ -579,6 +673,216 @@ def check_cross_attention(B=2, heads=8, d=40, seq=300, kv_seq=77, ctx_dim=768):
     return _stats(out, ref, f"cross attention d={d} seq={seq} kv={kv_seq}", 2e-2, 2e-2)
 
 
+# ----------------------------------------------------------------------------------------------------------- attention edges
+# Inputs chosen so that the data reaches what random scores never do: one dominant key per row at block and half-block
+# boundaries, block maxima that jump by more than the lazy (2^8) and redo (2^64) thresholds, rows whose scores all lie
+# far below zero or are all equal. fp64 reference with the maximum subtracted (attn_ref), bound comparator above.
+LOG2E = math.log2(math.e)
+EDGE_KV = (1, 16, 47, 48, 49, 95, 96, 97, 129, 7488)
+CROSS_QUERIES = 300   # two 256-query CTAs of the 40-wide kernel, three 128-query tiles of the others, ragged
+
+
+def _attn_where(idx):
+    bh, row, ch = idx
+    return {"image_head": bh, "query_row": row, "channel": ch, "query_tile_128": row // 128,
+            "warp_slice_32": (row % 128) // 32}
+
+
+def _attn_launch(q, k, v, d, scale, cross):
+    """flash_attn on q [heads, S, d], k / v [heads, kv, d] (bf16, one image): self-attention (S == kv) through one set of
+    head-split buffers, cross-attention through a separate key / value set. Returns out [heads, S, d]."""
+    heads, S, _ = q.shape
+    kv = k.shape[1]
+    qb = ops.alloc_qkv(1, heads, S, d, DEV)
+    kb = ops.alloc_kv(1, heads, kv, d, DEV) if cross else qb
+    assert cross or kv == S
+    qb["q"][:, :, :d] = q
+    kb["k"][:, :, :d] = k
+    kb["vt"][:, :d, :kv] = v.transpose(1, 2)
+    out = _empty((S, heads * d), dtype=bf16, device=DEV)
+    ops.flash_attn(qb["q"], kb["k"], kb["vt"], out, B=1, heads=heads, seq=S, head_dim=d, dpad=kb["dpad"],
+                   seq_pad=kb["seq_pad"], scale=scale, kv_seq=kv if cross else 0)
+    return out.view(S, heads, d).transpose(0, 1)
+
+
+def _bf16_scalar(x):
+    return float(torch.tensor(x).to(bf16))
+
+
+def needle_positions(kv):
+    """Key 0, the last key, both sides of the 48-key halves of the 40-wide kernel and of the 64- / 96-key block
+    boundaries, and both sides of the start of the ragged last block."""
+    pos = {0, kv - 1, 47, 48, 63, 64, 95, 96, 127, 128, 191, 192}
+    for blk in (64, 96):
+        last = (kv - 1) // blk * blk
+        pos |= {last - 1, last}
+    return sorted(p for p in pos if 0 <= p < kv)
+
+
+def needle_inputs(S, kv, d, margin, heads=2, seed=0):
+    """Row i of head h attends to key needle_positions(kv)[(i + h) % n]. Key j carries the bits of j as signs in its
+    first `bits` channels, the query the needle's signs times sigma: the needle scores sigma * bits, every other key at
+    least 2 sigma less, i.e. `margin` log2 units at scale d^-0.5. |V| in [1, 2). Returns q, k, v (bf16) and the needle
+    index of every (head, row)."""
+    g = _gen(seed)
+    bits = max(1, (kv - 1).bit_length())
+    assert bits <= d
+    scale = d ** -0.5
+    sigma = _bf16_scalar(margin / (2 * scale * LOG2E))
+    sign = ((torch.arange(kv)[:, None] >> torch.arange(bits)) & 1).float() * 2 - 1      # [kv, bits]
+    pos = torch.tensor(needle_positions(kv))
+    tgt = pos[(torch.arange(S)[None, :] + torch.arange(heads)[:, None]) % len(pos)]      # [heads, S]
+    q = torch.zeros((heads, S, d))
+    q[:, :, :bits] = sigma * sign[tgt]
+    k = torch.zeros((heads, kv, d))
+    k[:, :, :bits] = sign
+    v = torch.where(torch.rand((heads, kv, d), generator=g) < 0.5, -1.0, 1.0) * (1 + torch.rand((heads, kv, d), generator=g))
+    return q.to(bf16), k.to(bf16), v.to(bf16), tgt
+
+
+def check_attn_needles(d, cross):
+    """Needles on every boundary, margins of 7, 20, 40 and 100 log2 units. With the needle in a block j > 0, that
+    block's maximum exceeds the running reference by the margin when an earlier key is one sign flip away (needle 96,
+    key 32: the first block of every kernel, the same half in the 40-wide one): at 7, P up to 2^7 accumulates into O without a rescale (the lazy
+    threshold is 2^8); at 20 and 40, O is rescaled lazily; at 100, the block's exponentials are redone (> 2^64). From
+    20 up, the other keys weigh <= 13 * 2^-20, and the output must be the needle's V row to bf16 rounding."""
+    worst = 0.0
+    scale = d ** -0.5
+    for kv in EDGE_KV:
+        S = CROSS_QUERIES if cross else kv
+        for margin in (7.0, 20.0, 40.0, 100.0):
+            q, k, v, tgt = needle_inputs(S, kv, d, margin, seed=kv)
+            q, k, v = q.to(DEV), k.to(DEV), v.to(DEV)
+            out = _attn_launch(q, k, v, d, scale, cross)
+            ref, mag = attn_ref(q, k, v, scale)
+            name = f"attn needles d={d} {'cross' if cross else 'self'} S={S} kv={kv} margin={margin}"
+            worst = max(worst, _bound_stats(out, ref, mag, name, U_BF16, A_ATTN, where=_attn_where)["worst_ratio"])
+            if margin < 20:
+                continue
+            want = torch.gather(v, 1, tgt.to(DEV)[:, :, None].expand(-1, -1, d)).float()
+            off = (out.float() - want).abs() > U_BF16 * want.abs()
+            assert not off.any(), f"{name}: {int(off.sum())} outputs differ from the needle's V row by more than bf16 " \
+                                  f"rounding, first at {_attn_where(tuple(off.nonzero()[0].tolist()))}"
+    return {"name": f"attn needles d={d} cross={cross}", "worst_ratio": worst}
+
+
+def check_attn_const_v(d, cross):
+    """V constant along the keys: the output must be that constant to one bf16 ulp for any P, i.e. the numerator and the
+    row sum (the ones row of V^T at d = 40) see the same P. Peaked random scores (std ~6 log2 units)."""
+    worst = 0.0
+    scale = d ** -0.5
+    for kv in EDGE_KV:
+        S = CROSS_QUERIES if cross else kv
+        g = _gen(100 + kv)
+        q = (torch.randn((2, S, d), generator=g) * 4).to(bf16).to(DEV)
+        k = torch.randn((2, kv, d), generator=g).to(bf16).to(DEV)
+        c = (torch.where(torch.rand((2, 1, d), generator=g) < 0.5, -1.0, 1.0) *
+             (0.5 + 1.5 * torch.rand((2, 1, d), generator=g))).to(bf16).to(DEV)
+        v = c.expand(-1, kv, -1).contiguous()
+        out = _attn_launch(q, k, v, d, scale, cross)
+        ref, mag = attn_ref(q, k, v, scale)
+        name = f"attn constant V d={d} {'cross' if cross else 'self'} S={S} kv={kv}"
+        worst = max(worst, _bound_stats(out, ref, mag, name, U_BF16, A_ATTN, where=_attn_where)["worst_ratio"])
+        ulp = torch.exp2(torch.floor(torch.log2(c.float().abs())) - 7)
+        off = (out.float() - c.float()).abs() > ulp
+        assert not off.any(), f"{name}: {int(off.sum())} outputs more than one bf16 ulp from the constant, first at " \
+                              f"{_attn_where(tuple(off.nonzero()[0].tolist()))}"
+    return {"name": f"attn constant V d={d} cross={cross}", "worst_ratio": worst}
+
+
+def check_attn_flat(d, cross):
+    """Every score of a row far below zero (a common offset of -100 / -200 log2 units on scores of std ~1.4), and every
+    score of a row equal (all keys the same). Outputs finite and within the bound."""
+    worst = 0.0
+    scale = d ** -0.5
+    for kv in (1, 16, 47, 48, 49, 95, 96, 97, 300):
+        S = CROSS_QUERIES if cross else kv
+        for case in (-100.0, -200.0, "equal"):
+            g = _gen(200 + kv)
+            q = torch.randn((2, S, d), generator=g)
+            k = torch.randn((2, kv, d), generator=g)
+            if case == "equal":
+                k = k[:, :1].expand(-1, kv, -1)
+            else:   # one channel carries the offset: 8 * kb * scale * log2(e) = offset
+                q[:, :, d - 1] = 8.0
+                k[:, :, d - 1] = _bf16_scalar(case / (8.0 * scale * LOG2E))
+            q, k = q.to(bf16).to(DEV), k.contiguous().to(bf16).to(DEV)
+            v = torch.randn((2, kv, d), generator=g).to(bf16).to(DEV)
+            out = _attn_launch(q, k, v, d, scale, cross)
+            ref, mag = attn_ref(q, k, v, scale)
+            name = f"attn flat scores d={d} {'cross' if cross else 'self'} S={S} kv={kv} case={case}"
+            worst = max(worst, _bound_stats(out, ref, mag, name, U_BF16, A_ATTN, where=_attn_where)["worst_ratio"])
+    return {"name": f"attn flat scores d={d} cross={cross}", "worst_ratio": worst}
+
+
+def attn_random_inputs(S, kv, d, heads, spread, seed):
+    """q ~ N(0, spread^2), k, v ~ N(0, 1) in bf16: scores of std spread * log2(e) log2 units at scale d^-0.5."""
+    g = _gen(seed)
+    return tuple(torch.randn((heads, n, d), generator=g).mul(s).to(bf16)
+                 for n, s in ((S, spread), (kv, 1.0), (kv, 1.0)))
+
+
+def check_attention_bound(d, seq, heads=2, spread=4.0):
+    """Random self-attention against the fp64 reference with the bound comparator, at the largest shape of the plans
+    (d = 40, 7 488 tokens): the data tests/test_bound_controls.py shows the comparator's sensitivity on."""
+    q, k, v = (t.to(DEV) for t in attn_random_inputs(seq, seq, d, heads, spread, 300 + d))
+    out = _attn_launch(q, k, v, d, d ** -0.5, False)
+    ref, mag = attn_ref(q, k, v, d ** -0.5)
+    return _bound_stats(out, ref, mag, f"attn bound d={d} seq={seq} spread={spread}", U_BF16, A_ATTN, where=_attn_where)
+
+
+# ----------------------------------------------------------------------------------------------------------- norm cancellation
+def cancellation_input(shape, seed):
+    """x [n, m, groups, cpg]: every (n, group) has a mean of 16, 32 or 64 times its spread (cycling over the groups,
+    random sign), spread in [0.5, 2). In bf16 the 64x groups still resolve spread / 2."""
+    n, m, groups, cpg = shape
+    g = _gen(seed)
+    spread = 0.5 + 1.5 * torch.rand((n, 1, groups, 1), generator=g)
+    ratio = torch.tensor([16.0, 32.0, 64.0]).repeat(groups)[:groups].view(1, 1, groups, 1)
+    sign = torch.where(torch.rand((n, 1, groups, 1), generator=g) < 0.5, -1.0, 1.0)
+    return ((sign * ratio + torch.randn(shape, generator=g)) * spread).to(bf16)
+
+
+def _launched_kernels(fn):
+    """Names of the CUDA kernels `fn` launches (torch.profiler, CUDA activity only)."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return {e.name for e in prof.events()}
+
+
+GN_KERNELS = ("gn_fused_kernel", "gn_cluster_kernel", "gn_stats_kernel")
+
+
+def check_groupnorm_cancel(c1, c2, HW, B, silu, kernel, eps=1e-5):
+    """`kernel`: the GroupNorm kernel the shape must select (gn_fused_kernel, the cooperative two-sweep kernel, or
+    gn_cluster_kernel), so that a change of the selection cannot move this coverage silently."""
+    C = c1 + c2
+    x = cancellation_input((B, HW, 32, C // 32), 60 + B).view(B, HW, C).to(DEV)
+    x1 = x[..., :c1].contiguous()
+    x2 = x[..., c1:].contiguous() if c2 else None
+    g, b = _randn((C,), 8) * 0.2 + 1, _randn((C,), 9) * 0.1
+    out = _empty((B, HW, C), dtype=bf16, device=DEV)
+    stats = ops.gn_scratch(B, 32, DEV)
+    names = _launched_kernels(lambda: ops.groupnorm(x1, g, b, out, stats, x2=x2, groups=32, eps=eps, silu=silu))
+    ran = [k for k in GN_KERNELS if any(k in n for n in names)]
+    assert ran == [kernel], f"groupnorm B={B} HW={HW} C={C}: expected {kernel}, launched {ran} ({sorted(names)})"
+    assert int(stats[-2 * B:].view(torch.int32).abs().sum()) == 0, "groupnorm left its barrier counters non-zero"
+    ref, mag = norm_ref(x, g, b, eps, groups=32, silu=silu)
+    return _bound_stats(out, ref, mag, f"groupnorm cancellation c1={c1} c2={c2} HW={HW} B={B} silu={silu}", U_BF16,
+                        A_NORM, where=lambda i: {"image": i[0], "pixel": i[1], "group": i[2] // (C // 32)})
+
+
+def check_layernorm_cancel(C, rows):
+    x = cancellation_input((rows, 1, 1, C), 70 + C).view(rows, C).to(DEV)
+    g, b = _randn((C,), 4) * 0.2 + 1, _randn((C,), 5) * 0.1
+    out = _empty_like(x)
+    ops.layernorm(x, g, b, out, 1e-5)
+    ref, mag = norm_ref(x, g, b, 1e-5)
+    return _bound_stats(out, ref, mag, f"layernorm cancellation C={C} rows={rows}", U_BF16, A_NORM)
+
+
 # ----------------------------------------------------------------------------------------------------------- integer tail
 def check_logits_to_ids(up=2):
     B, h, w, C = 2, 24, 78, 128
@@ -795,6 +1099,24 @@ CHECKS = {
     "cross_attn_40_kv128_long": lambda: check_cross_attention(1, 8, 40, 7488, 128),
     "cross_attn_80_kv257": lambda: check_cross_attention(2, 8, 80, 468, 257, 1024),
     "cross_attn_160_kv16": lambda: check_cross_attention(2, 8, 160, 120, 16, 64),
+    **{f"attn_{kind}_{d}_{'cross' if cross else 'self'}": (lambda f=f, d=d, cross=cross: f(d, cross))
+       for kind, f in (("needles", check_attn_needles), ("const_v", check_attn_const_v), ("flat", check_attn_flat))
+       for d in (40, 80, 160) for cross in (False, True)},
+    "attn_bound_40_level0": lambda: check_attention_bound(40, 7488),
+    "attn_bound_80": lambda: check_attention_bound(80, 1872),
+    "attn_bound_160": lambda: check_attention_bound(160, 468),
+    # mean 16-64x the spread: E[x^2] - mean^2 cancellation, in both GroupNorm kernels (each entry asserts which one ran),
+    # concat inputs, SiLU on and off
+    "groupnorm_cancel_L0_b8_coop": lambda: check_groupnorm_cancel(320, 0, 7488, 8, True, "gn_fused_kernel"),
+    "groupnorm_cancel_L0_b8_coop_nosilu": lambda: check_groupnorm_cancel(320, 0, 7488, 8, False, "gn_fused_kernel"),
+    "groupnorm_cancel_L1_b8_coop": lambda: check_groupnorm_cancel(640, 0, 1872, 8, True, "gn_fused_kernel"),
+    "groupnorm_cancel_L0_b1_cluster": lambda: check_groupnorm_cancel(320, 0, 7488, 1, False, "gn_cluster_kernel"),
+    "groupnorm_cancel_960cat_b2_cluster": lambda: check_groupnorm_cancel(640, 320, 1872, 2, True, "gn_cluster_kernel"),
+    "groupnorm_cancel_L3_2560cat_b8_cluster_nosilu":
+        lambda: check_groupnorm_cancel(1280, 1280, 120, 8, False, "gn_cluster_kernel"),
+    "layernorm_cancel_320": lambda: check_layernorm_cancel(320, 20000),
+    "layernorm_cancel_640": lambda: check_layernorm_cancel(640, 5000),
+    "layernorm_cancel_1280": lambda: check_layernorm_cancel(1280, 2000),
     "logits_to_ids_up2": check_logits_to_ids,
     "logits_to_ids_up1": lambda: check_logits_to_ids(1),
     "segment_filter_boundaries": check_segment_filter_boundaries,

@@ -299,7 +299,7 @@ flash_attn40_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
           mx1 = fmax3(mx1, __uint_as_float(sv[i + 2]), __uint_as_float(sv[i + 3]));
         }
         m = fmaxf(mx0, mx1) * p.scale_log2;
-        if (m == -INFINITY) m = 0.f;  // this half has no key at all (seq <= 48): P = 0, l = 0, the merge ignores it
+        if (m == -INFINITY) m = 0.f;  // this half has no key at all (kv_seq <= 48): P = 0, l = 0 (see the merge)
         m_seen = m;
       } else {
         const bool need = m_seen - m > kLazy;
@@ -336,10 +336,12 @@ flash_attn40_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 #pragma unroll
       for (int i = 0; i < kDN; ++i) o_acc[i] = __uint_as_float(v[i]);
     }
-    // merge the two halves of a row: half 1 publishes (m, l, O) through shared memory, half 0 combines
+    // merge the two halves of a row: half 1 publishes (m, l, O) through shared memory, half 0 combines. Half 0 always
+    // has a key; half 1 has none when kv_seq <= 48 and then enters with m = -inf, i.e. weight a1 = 0, a0 = 1. (Its
+    // placeholder m = 0 would give a0 = 2^(m0 - 0) = 0 and 1 / 0 for a row whose scores all lie below -126 log2 units.)
     float* mg = sMerge + (g * 128 + r) * kMergeStride;
     if (h == 1) {
-      mg[0] = m;
+      mg[0] = p.kv_seq > kHalf ? m : -INFINITY;
       mg[1] = o_acc[kD];
 #pragma unroll
       for (int c = 0; c < kD; ++c) mg[2 + c] = o_acc[c];
