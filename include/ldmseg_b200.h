@@ -250,6 +250,22 @@ int ldm_ddim_step_clip(const float* eps_uncond, const float* eps_text, float gui
                        const float* coef, const int32_t* t_index, float* prev_sample, float* pred_x0, int64_t n,
                        float clip_sample_range, int32_t use_clipped_model_output, ldm_stream_t stream);
 
+/* DPM-Solver++ multistep update (algorithm_type "dpmsolver++", solver_type "midpoint", epsilon prediction, solver
+ * order 1 or 2), fp32, bit-exact with the same formulas in torch eager on the CPU (round-to-nearest, this op order):
+ *   x0   = (sample - sig_i * eps) / alpha_i
+ *   prev = A * sample - Bc * x0                                  (order 1)
+ *   prev = (A * sample - Bc * x0) - hb * (c * (x0 - x0_prev))    (order 2)
+ * with A = sig_{i+1} / sig_i, Bc = alpha_{i+1} * (exp(-h) - 1), h = lam_{i+1} - lam_i, c = 1 / r0,
+ * r0 = (lam_i - lam_{i-1}) / h, hb = 0.5 * Bc, and per sigma alpha = 1 / sqrt(sigma^2 + 1), sig = sigma * alpha,
+ * lam = log(alpha) - log(sig). The host builds these scalars: coef is a device f32 [steps, 8] table, row i =
+ * {sig_i, alpha_i, A, Bc, c, hb, order (1.0 or 2.0), 0}, selected by the DEVICE int32 *step_index (no host sync).
+ * eps_text != NULL: eps = eps_uncond + guidance_scale * (eps_text - eps_uncond) first, as ldm_ddim_step_cfg.
+ * x0 is written to x0_prev in place (read first when order == 2); prev_sample may alias sample. No argument but
+ * eps_text may be NULL. */
+int ldm_dpmpp_step(const float* eps_uncond, const float* eps_text, float guidance_scale, const float* sample,
+                   const float* coef, const int32_t* step_index, float* prev_sample, float* x0_prev, int64_t n,
+                   ldm_stream_t stream);
+
 /* Layout helpers (NHWC bf16). */
 int ldm_upsample_nearest(const void* x, void* out, int32_t B, int32_t h, int32_t w, int32_t C, int32_t oh,
                          int32_t ow, ldm_stream_t stream); /* F.interpolate(mode="nearest") */

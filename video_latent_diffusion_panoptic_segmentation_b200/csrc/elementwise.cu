@@ -1,4 +1,4 @@
-// Small HBM-/latency-bound kernels of the sampler loop: DDIM update, timestep sinusoid + GEMV chain, the
+// Small HBM-/latency-bound kernels of the sampler loop: DDIM and DPM-Solver++ updates, timestep sinusoid + GEMV chain, the
 // few-channel 3x3 convs at the ends of the UNet / seg-AE (fused with concat+cast), nearest upsample, stride-2 im2col.
 #include "common.cuh"
 #include "host_util.h"
@@ -56,6 +56,60 @@ __global__ void ddim_step_kernel(const float* __restrict__ eps, const float* __r
     if (reclip_eps) e = __fdiv_rn(__fsub_rn(sample[i], __fmul_rn(s_at, p0)), s1m_at);
     if (prev) prev[i] = __fadd_rn(__fmul_rn(s_ap, p0), __fmul_rn(s1m_ap, e));
     if (x0out) x0out[i] = p0;
+  }
+}
+
+// ---------------------------------------------------------------- DPM-Solver++ (2M, midpoint) update
+// Row *step_index of `coef` (ldmseg/schedulers/dpm_solver.py) holds {sig_i, alpha_i, A, Bc, c, hb, order, 0}:
+//   x0 = (x - sig_i * eps) / alpha_i;  prev = A * x - Bc * x0  [ - hb * (c * (x0 - x0_prev)) when order == 2 ]
+// in that op order with round-to-nearest intrinsics, as ddim_step_kernel. x0 replaces x0_prev in place (the same thread
+// reads and writes each element); `prev` may alias `sample`.
+constexpr int kDpmCoefCols = 8;
+__global__ void dpmpp_step_kernel(const float* __restrict__ eps, const float* __restrict__ eps_text, float guidance,
+                                  const float* sample, const float* __restrict__ coef,
+                                  const int32_t* __restrict__ step_index, float* prev, float* x0_prev, long long n) {
+  const float* row = coef + (long long)__ldg(step_index) * kDpmCoefCols;
+  const float sig = __ldg(row + 0), alpha = __ldg(row + 1), A = __ldg(row + 2), Bc = __ldg(row + 3);
+  const float c = __ldg(row + 4), hb = __ldg(row + 5);
+  const bool second = __ldg(row + 6) > 1.5f;
+  const long long nv = n / 4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+    const float4 e = __ldg(reinterpret_cast<const float4*>(eps) + i);
+    const float4 x = reinterpret_cast<const float4*>(sample)[i];
+    float ev[4] = {e.x, e.y, e.z, e.w};
+    if (eps_text) {
+      const float4 t = __ldg(reinterpret_cast<const float4*>(eps_text) + i);
+      const float tv[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) ev[j] = __fadd_rn(ev[j], __fmul_rn(guidance, __fsub_rn(tv[j], ev[j])));
+    }
+    const float xv[4] = {x.x, x.y, x.z, x.w};
+    float qv[4] = {0.f, 0.f, 0.f, 0.f};
+    if (second) {
+      const float4 q = reinterpret_cast<const float4*>(x0_prev)[i];
+      qv[0] = q.x; qv[1] = q.y; qv[2] = q.z; qv[3] = q.w;
+    }
+    float p0[4], pv[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      p0[j] = __fdiv_rn(__fsub_rn(xv[j], __fmul_rn(sig, ev[j])), alpha);
+      pv[j] = __fsub_rn(__fmul_rn(A, xv[j]), __fmul_rn(Bc, p0[j]));
+      if (second) pv[j] = __fsub_rn(pv[j], __fmul_rn(hb, __fmul_rn(c, __fsub_rn(p0[j], qv[j]))));
+    }
+    reinterpret_cast<float4*>(prev)[i] = make_float4(pv[0], pv[1], pv[2], pv[3]);
+    reinterpret_cast<float4*>(x0_prev)[i] = make_float4(p0[0], p0[1], p0[2], p0[3]);
+  }
+  // tail
+  for (long long i = nv * 4 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+       i += (long long)gridDim.x * blockDim.x) {
+    float e = eps[i];
+    if (eps_text) e = __fadd_rn(e, __fmul_rn(guidance, __fsub_rn(eps_text[i], e)));
+    const float x = sample[i];
+    const float p0 = __fdiv_rn(__fsub_rn(x, __fmul_rn(sig, e)), alpha);
+    float p = __fsub_rn(__fmul_rn(A, x), __fmul_rn(Bc, p0));
+    if (second) p = __fsub_rn(p, __fmul_rn(hb, __fmul_rn(c, __fsub_rn(p0, x0_prev[i]))));
+    prev[i] = p;
+    x0_prev[i] = p0;
   }
 }
 
@@ -293,6 +347,23 @@ extern "C" int ldm_ddim_step_clip(const float* eps_uncond, const float* eps_text
                                                                             use_clipped_model_output != 0);
   count_launch();
   return check_launch("ddim_step_kernel");
+}
+
+extern "C" int ldm_dpmpp_step(const float* eps_uncond, const float* eps_text, float guidance_scale, const float* sample,
+                              const float* coef, const int32_t* step_index, float* prev_sample, float* x0_prev, int64_t n,
+                              ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(eps_uncond && sample && coef && step_index && prev_sample && x0_prev, LDM_ERR_BAD_ARG,
+              "ldm_dpmpp_step: null arg");
+  LDM_REQUIRE(n > 0, LDM_ERR_BAD_SHAPE, "ldm_dpmpp_step: n=%lld", (long long)n);
+  LDM_REQUIRE(((uintptr_t)eps_uncond | (uintptr_t)eps_text | (uintptr_t)sample | (uintptr_t)prev_sample |
+               (uintptr_t)x0_prev) % 16 == 0,
+              LDM_ERR_ALIGNMENT, "ldm_dpmpp_step: pointers must be 16-byte aligned");
+  dpmpp_step_kernel<<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(eps_uncond, eps_text, guidance_scale,
+                                                                             sample, coef, step_index, prev_sample,
+                                                                             x0_prev, n);
+  count_launch();
+  return check_launch("dpmpp_step_kernel");
 }
 
 extern "C" int ldm_timestep_sinusoid(const int64_t* timesteps, const int32_t* t_index, const float* freqs, float* out,

@@ -23,6 +23,28 @@ class DDIMNoiseSchedulerOutput(OutputDict):
     pred_original_sample: Optional[torch.Tensor] = None
 
 
+def betas_for_alpha_bar(num_diffusion_timesteps, max_beta=0.999) -> torch.Tensor:
+    def alpha_bar(t):
+        return math.cos((t + 0.008) / 1.008 * math.pi / 2) ** 2
+    n = num_diffusion_timesteps
+    return torch.tensor([min(1 - alpha_bar((i + 1) / n) / alpha_bar(i / n), max_beta) for i in range(n)],
+                        dtype=torch.float32)
+
+
+def make_betas(beta_schedule: str, beta_start: float, beta_end: float, num_train_timesteps: int,
+               owner=None) -> torch.Tensor:
+    """The beta schedule (:51-61) in fp32, shared by every scheduler of the package."""
+    if beta_schedule == "linear":
+        return torch.linspace(beta_start, beta_end, num_train_timesteps, dtype=torch.float32)
+    if beta_schedule == "scaled_linear":
+        return torch.linspace(beta_start ** 0.5, beta_end ** 0.5, num_train_timesteps, dtype=torch.float32) ** 2
+    if beta_schedule == "squaredcos_cap_v2":
+        return betas_for_alpha_bar(num_train_timesteps)
+    if beta_schedule == "sigmoid":
+        return torch.sigmoid(torch.linspace(-6, 6, num_train_timesteps)) * (beta_end - beta_start) + beta_start
+    raise NotImplementedError(f"{beta_schedule} does is not implemented for {owner}")
+
+
 class DDIMNoiseScheduler(object):
     def __init__(self, num_train_timesteps: int = 1000, beta_start: float = 0.0001, beta_end: float = 0.02,
                  beta_schedule: str = "linear", clip_sample: bool = True, set_alpha_to_one: bool = True,
@@ -30,17 +52,7 @@ class DDIMNoiseScheduler(object):
                  dynamic_thresholding_ratio: float = 0.995, clip_sample_range: float = 1.0,
                  sample_max_value: float = 1.0, weight: str = "none", max_snr: float = 5.0,
                  device: Union[str, torch.device] = None, verbose: bool = True):
-        if beta_schedule == "linear":
-            self.betas = torch.linspace(beta_start, beta_end, num_train_timesteps, dtype=torch.float32)
-        elif beta_schedule == "scaled_linear":
-            self.betas = torch.linspace(beta_start ** 0.5, beta_end ** 0.5, num_train_timesteps,
-                                        dtype=torch.float32) ** 2
-        elif beta_schedule == "squaredcos_cap_v2":
-            self.betas = self.get_betas_for_alpha_bar(num_train_timesteps)
-        elif beta_schedule == "sigmoid":
-            self.betas = torch.sigmoid(torch.linspace(-6, 6, num_train_timesteps)) * (beta_end - beta_start) + beta_start
-        else:
-            raise NotImplementedError(f"{beta_schedule} does is not implemented for {self.__class__}")
+        self.betas = make_betas(beta_schedule, beta_start, beta_end, num_train_timesteps, owner=self.__class__)
         self.alphas = 1.0 - self.betas
         self.alphas_cumprod = torch.cumprod(self.alphas, dim=0)
         self.final_alpha_cumprod = torch.tensor(1.0) if set_alpha_to_one else self.alphas_cumprod[0]
@@ -76,11 +88,7 @@ class DDIMNoiseScheduler(object):
             self.weights = torch.ones_like(snr)
 
     def get_betas_for_alpha_bar(self, num_diffusion_timesteps, max_beta=0.999) -> torch.Tensor:
-        def alpha_bar(t):
-            return math.cos((t + 0.008) / 1.008 * math.pi / 2) ** 2
-        n = num_diffusion_timesteps
-        return torch.tensor([min(1 - alpha_bar((i + 1) / n) / alpha_bar(i / n), max_beta) for i in range(n)],
-                            dtype=torch.float32)
+        return betas_for_alpha_bar(num_diffusion_timesteps, max_beta)
 
     # ------------------------------------------------------------------ inference timesteps (:119-136)
     def set_timesteps_inference(self, num_inference_steps: int, device: Union[str, torch.device] = None, tmin: int = 0):

@@ -4,7 +4,7 @@
 
 Data flow of one batch, all on the GPU:
   noise (CPU generator, as the reference) -> H2D
-  T x [ UNet CUDA graph (concat+cast fused into conv_in)  ->  fused DDIM update kernel ]      no host sync inside
+  T x [ UNet CUDA graph (concat+cast fused into conv_in)  ->  fused DDIM (or DPM-Solver++) update ]      no host sync inside
   seg-AE decoder (NHWC fp32 logits at 4h x 4w)
   fused bilinear x2 + argmax + softmax-max threshold + per-class areas  ->  merge filter  ->  int32 panoptic ids
   PQ / DVPQ statistics from joint id histograms
@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from ..evaluations.cityscapes_pap_eval import CityscapesPanopticEvaluator
+from ..schedulers import DPMSolverMultistepScheduler
 from ..utils import color_map, get_world_size, is_dist_avail_and_initialized, is_main_process
 from ... import _lib as L
 from ... import ops
@@ -95,9 +96,10 @@ class TrainerDiffusion:
         return latents * scaling_factor, latents_mean * scaling_factor
 
     # ------------------------------------------------------------------ sample (:1048-1173)
-    def _loop_state(self, B, h, w, multiplier=1, ctx_len=None):
+    def _loop_state(self, B, h, w, multiplier=1, ctx_len=None, dpm=False):
         """Static buffers + UNet plan for the DDIM loop at this shape (built once, reused for every batch). With
-        classifier-free guidance (multiplier 2) the UNet runs on the doubled batch [uncond | text] (:1129,1126)."""
+        classifier-free guidance (multiplier 2) the UNet runs on the doubled batch [uncond | text] (:1129,1126).
+        dpm: also the x0_prev buffer of the DPM-Solver++ loop (same plan)."""
         key = (B, h, w, self.self_condition, multiplier, ctx_len)
         st = self._loop.get(key)
         if st is None:
@@ -110,6 +112,8 @@ class TrainerDiffusion:
                 parts.append(st["cond"])
             st["plan"] = self.unet_model._get_plan(n, h, w, 4 * len(parts), parts=parts, ctx_len=ctx_len)
             self._loop[key] = st
+        if dpm and "x0_prev" not in st:  # the DPM-Solver++ update's previous x0 prediction
+            st["x0_prev"] = torch.empty((B, 4, h, w), dtype=f32, device=self.device)
         return st
 
     def norm_resize_images(self, x):
@@ -156,6 +160,13 @@ class TrainerDiffusion:
         if scheduler is None:
             scheduler = self.noise_scheduler
             scheduler.set_timesteps_inference(num_inference_steps)
+        dpm = isinstance(scheduler, DPMSolverMultistepScheduler)
+        if not dpm and not (hasattr(scheduler, "coef_table") and hasattr(scheduler, "clip_range")):
+            raise NotImplementedError(f"sample: scheduler {type(scheduler).__name__} is not supported: pass this "
+                                      "package's DDIMNoiseScheduler or DPMSolverMultistepScheduler")
+        if dpm and self.self_condition:
+            raise NotImplementedError("self_condition with DPMSolverMultistepScheduler: the condition is the step's "
+                                      "pred_original_sample (:1152-1153), which the DPM-Solver step output does not carry")
         if rgb_latents is None:
             raise NotImplementedError("unconditional sampling (rgb_latents=None) is not on the eval path")
         if repeat_noise is None:
@@ -177,7 +188,7 @@ class TrainerDiffusion:
             raise NotImplementedError("self_condition with a text encoder: the reference concatenates a doubled batch "
                                       "with an undoubled condition (:1134-1136,1152-1153) and fails")
         B = batch_size
-        st = self._loop_state(B, h, w, multiplier, ctx_len=None if ctx is None else ctx.shape[1])
+        st = self._loop_state(B, h, w, multiplier, ctx_len=None if ctx is None else ctx.shape[1], dpm=dpm)
         lat_all, plan = st["latents"], st["plan"]
         latents = lat_all[:B]
         latents.copy_(noise.to(dev, non_blocking=True))           # H2D (:1095)
@@ -192,6 +203,9 @@ class TrainerDiffusion:
         if ctx is not None:  # k / v of every attn2 layer are projected once here, not once per step
             unet.set_context(plan, ctx if uncond is None else torch.cat([uncond, ctx]))   # (:1120)
         timesteps = scheduler.timesteps.to(dev)
+        if dpm:
+            return self._dpm_loop(st, latents, B, multiplier, scheduler, timesteps, guidance_scale, return_all_latents,
+                                  original_noise)
         coef = scheduler.coef_table(dev)
         clip = scheduler.clip_range()  # scheduler.step's clip_sample (:1152-1154 calls it with its defaults)
         all_latents = []
@@ -220,6 +234,34 @@ class TrainerDiffusion:
             return torch.cat(all_latents, dim=0)
         out = latents.clone()
         if repeat_noise:
+            return out, original_noise
+        return out
+
+    def _dpm_loop(self, st, latents, B, multiplier, scheduler, timesteps, guidance_scale, return_all_latents,
+                  original_noise):
+        """The sampler loop of sample() with a DPMSolverMultistepScheduler: the same UNet graph, then one fused
+        DPM-Solver++ update (guidance included) per step. Its last step goes to sigma = 0, where prev equals x0: the
+        latents end as the final x0 prediction, as DDIM's last step leaves them."""
+        dev, lat_all, plan = self.device, st["latents"], st["plan"]
+        coef, steps = scheduler.coef_table(dev), scheduler.step_index_table(dev)
+        x0_prev = st["x0_prev"]
+        all_latents = []
+        for i in range(timesteps.numel()):
+            plan.timestep.copy_(timesteps[i:i + 1])
+            if multiplier > 1:
+                lat_all[B:].copy_(latents)
+            if plan.graph is not None:
+                plan.graph.replay()
+            else:
+                self.unet_model._run_plan(plan)
+            ops.dpmpp_step(plan.out[:B], latents, coef, steps[i:i + 1], prev_sample=latents, x0_prev=x0_prev,
+                           eps_text=plan.out[B:] if multiplier > 1 else None, guidance_scale=guidance_scale)
+            if return_all_latents:
+                all_latents.append(latents.clone())
+        if return_all_latents:
+            return torch.cat(all_latents, dim=0)
+        out = latents.clone()
+        if original_noise is not None:
             return out, original_noise
         return out
 

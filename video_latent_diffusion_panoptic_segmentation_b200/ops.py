@@ -291,6 +291,24 @@ def ddim_step(eps, sample, coef, t_index, prev_sample=None, pred_x0=None, eps_te
                                        int(bool(use_clipped_model_output)), _stream()), "ldm_ddim_step_clip")
 
 
+def dpmpp_step(eps, sample, coef, step_index, prev_sample, x0_prev, eps_text=None, guidance_scale=0.0):
+    """DPM-Solver++ update with the scalars of row *step_index of coef (f32 [steps, 8], DPMSolverMultistepScheduler):
+    prev_sample <- solver step of sample, x0_prev <- this step's x0 (read first on second-order rows). eps_text given:
+    classifier-free guidance first, as ddim_step. prev_sample may be sample."""
+    for t, n in ((eps, "eps"), (sample, "sample"), (coef, "coef"), (prev_sample, "prev"), (x0_prev, "x0_prev"),
+                 (eps_text, "eps_text")):
+        _chk(t, f32, n)
+    _chk(step_index, i32, "step_index")
+    n = sample.numel()
+    for t, name in ((eps, "eps"), (prev_sample, "prev"), (x0_prev, "x0_prev"), (eps_text, "eps_text")):
+        if t is not None and t.numel() != n:
+            raise L.LdmError(f"dpmpp_step: {name} has {t.numel()} elements, sample {n}")
+    if coef.dim() != 2 or coef.shape[1] != 8 or step_index.numel() != 1:
+        raise L.LdmError("dpmpp_step: coef must be [steps, 8] and step_index one int32 element")
+    L.check(L.lib().ldm_dpmpp_step(_p(eps), _p(eps_text), float(guidance_scale), _p(sample), _p(coef), _p(step_index),
+                                   _p(prev_sample), _p(x0_prev), n, _stream()), "ldm_dpmpp_step")
+
+
 def upsample_nearest(x, out):
     _chk(x, bf16, "x"); _chk(out, bf16, "out")
     B, h, w, Cc = x.shape
