@@ -266,6 +266,30 @@ int ldm_dpmpp_step(const float* eps_uncond, const float* eps_text, float guidanc
                    const float* coef, const int32_t* step_index, float* prev_sample, float* x0_prev, int64_t n,
                    ldm_stream_t stream);
 
+/* UniPC multistep update (predict_x0, solver_type "bh2", epsilon prediction, solver order 1, 2 or 3): the corrector
+ * UniC of the previous step's result and the predictor UniP to the next sigma in one launch, fp32, bit-exact with the
+ * same formulas in torch eager on the CPU (round-to-nearest, this op order; oracle/unipc_oracle.py states it in full):
+ *   m    = (sample - sig_i * eps) / alpha_i
+ *   S    = rho_m * (m - m1)                                                           (corrector order 1)
+ *   S    = ((rho_1 * ((m2 - m1) / r_1)) [+ rho_2 * ((m3 - m1) / r_2)]) + rho_m * (m - m1)     (order 2 [3])
+ *   xc   = (A * last - Phi * m1) - Bh * S                          (xc = sample when the corrector is off)
+ *   prev = A' * xc - Phi' * m                                                         (predictor order 1)
+ *   prev = (A' * xc - Phi' * m) - Bh' * ((rho'_1 * ((m1 - m) / r'_1)) [+ rho'_2 * ((m2 - m) / r'_2)])  (order 2 [3])
+ *   last <- xc;  m3 <- m2, m2 <- m1, m1 <- m
+ * Per sigma alpha = 1 / sqrt(sigma^2 + 1), sig = sigma * alpha, lam = log(alpha) - log(sig); an update from index a to
+ * t at order q has h = lam_t - lam_a, phi = B = expm1(-h), A = sig_t / sig_a, Phi = alpha_t * phi, Bh = alpha_t * B,
+ * r_k = (lam_{a-k} - lam_a) / h, and rho from the UniPC linear system (0.5 at predictor order 2 and corrector order 1).
+ * The corrector of step i updates a = i - 1 -> t = i; the predictor a = i -> t = i + 1. The host builds the scalars:
+ * coef is a device f32 [steps, 20] table, row i = {sig_i, alpha_i, p, q, A', Phi', Bh', r'_1, r'_2, rho'_1, rho'_2,
+ * A, Phi, Bh, r_1, r_2, rho_1, rho_2, rho_m, 0} with p the predictor order (1..3) and q the corrector order (0: off),
+ * selected by the DEVICE int32 *step_index (no host sync). eps_text != NULL: eps = eps_uncond + guidance_scale *
+ * (eps_text - eps_uncond) first, as ldm_ddim_step_cfg. m1 .. m_order are the previous x0 predictions (m1 the newest),
+ * updated in place; m_k with k > solver_order is not touched and may be NULL. prev_sample may alias sample; last,
+ * m1, m2, m3 alias nothing. Every element is read before it is written by the same thread. */
+int ldm_unipc_step(const float* eps_uncond, const float* eps_text, float guidance_scale, const float* sample,
+                   const float* coef, const int32_t* step_index, float* prev_sample, float* last, float* m1, float* m2,
+                   float* m3, int32_t solver_order, int64_t n, ldm_stream_t stream);
+
 /* Layout helpers (NHWC bf16). */
 int ldm_upsample_nearest(const void* x, void* out, int32_t B, int32_t h, int32_t w, int32_t C, int32_t oh,
                          int32_t ow, ldm_stream_t stream); /* F.interpolate(mode="nearest") */

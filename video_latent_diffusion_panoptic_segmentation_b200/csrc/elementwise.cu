@@ -1,5 +1,6 @@
-// Small HBM-/latency-bound kernels of the sampler loop: DDIM and DPM-Solver++ updates, timestep sinusoid + GEMV chain, the
-// few-channel 3x3 convs at the ends of the UNet / seg-AE (fused with concat+cast), nearest upsample, stride-2 im2col.
+// Small HBM-/latency-bound kernels of the sampler loop: DDIM, DPM-Solver++ and UniPC updates, timestep sinusoid +
+// GEMV chain, the few-channel 3x3 convs at the ends of the UNet / seg-AE (fused with concat+cast), nearest upsample,
+// stride-2 im2col.
 #include "common.cuh"
 #include "host_util.h"
 
@@ -110,6 +111,114 @@ __global__ void dpmpp_step_kernel(const float* __restrict__ eps, const float* __
     if (second) p = __fsub_rn(p, __fmul_rn(hb, __fmul_rn(c, __fsub_rn(p0, x0_prev[i]))));
     prev[i] = p;
     x0_prev[i] = p0;
+  }
+}
+
+// ---------------------------------------------------------------- UniPC (bh2, data prediction) update
+// Row *step_index of `coef` (ldmseg/schedulers/unipc.py, include/ldmseg_b200.h) holds the scalars of the corrector of
+// the previous step's result and of the predictor to the next sigma; the op order is that of oracle/unipc_oracle.py,
+// with round-to-nearest intrinsics as ddim_step_kernel. Each thread owns its elements: it reads sample, last and the
+// history m1..mQ of an element before it writes prev (which may alias sample), last and the shifted history.
+constexpr int kUniPCCoefCols = 20;
+struct UniPCRow {
+  float sig, alpha;
+  int p, q;                                  // predictor order 1..3, corrector order 0 (off) .. 3
+  float Ap, Pp, Bp, rp1, rp2, rhop1, rhop2;  // predictor: a = i -> t = i + 1
+  float Ac, Pc, Bc, rc1, rc2, rhoc1, rhoc2, rhocm;  // corrector: a = i - 1 -> t = i
+};
+
+__device__ __forceinline__ UniPCRow unipc_row(const float* __restrict__ coef, const int32_t* __restrict__ step_index) {
+  const float* r = coef + (long long)__ldg(step_index) * kUniPCCoefCols;
+  UniPCRow c;
+  c.sig = __ldg(r + 0); c.alpha = __ldg(r + 1);
+  c.p = __float2int_rn(__ldg(r + 2)); c.q = __float2int_rn(__ldg(r + 3));
+  c.Ap = __ldg(r + 4); c.Pp = __ldg(r + 5); c.Bp = __ldg(r + 6); c.rp1 = __ldg(r + 7); c.rp2 = __ldg(r + 8);
+  c.rhop1 = __ldg(r + 9); c.rhop2 = __ldg(r + 10);
+  c.Ac = __ldg(r + 11); c.Pc = __ldg(r + 12); c.Bc = __ldg(r + 13); c.rc1 = __ldg(r + 14); c.rc2 = __ldg(r + 15);
+  c.rhoc1 = __ldg(r + 16); c.rhoc2 = __ldg(r + 17); c.rhocm = __ldg(r + 18);
+  return c;
+}
+
+// One element: e is the (guided) noise prediction, x the sample, last the corrected sample of the previous step and
+// h[0..2] = m1..m3. Returns prev; last and h are updated in place (h[k] for k >= the history length is scratch).
+__device__ __forceinline__ float unipc_elem(const UniPCRow& c, float e, float x, float& last, float (&h)[3]) {
+  const float m = __fdiv_rn(__fsub_rn(x, __fmul_rn(c.sig, e)), c.alpha);
+  float xc = x;
+  if (c.q > 0) {
+    float s = __fmul_rn(c.rhocm, __fsub_rn(m, h[0]));
+    if (c.q > 1) {
+      float d = __fmul_rn(c.rhoc1, __fdiv_rn(__fsub_rn(h[1], h[0]), c.rc1));
+      if (c.q > 2) d = __fadd_rn(d, __fmul_rn(c.rhoc2, __fdiv_rn(__fsub_rn(h[2], h[0]), c.rc2)));
+      s = __fadd_rn(d, s);
+    }
+    xc = __fsub_rn(__fsub_rn(__fmul_rn(c.Ac, last), __fmul_rn(c.Pc, h[0])), __fmul_rn(c.Bc, s));
+  }
+  float prev = __fsub_rn(__fmul_rn(c.Ap, xc), __fmul_rn(c.Pp, m));
+  if (c.p > 1) {
+    float s = __fmul_rn(c.rhop1, __fdiv_rn(__fsub_rn(h[0], m), c.rp1));
+    if (c.p > 2) s = __fadd_rn(s, __fmul_rn(c.rhop2, __fdiv_rn(__fsub_rn(h[1], m), c.rp2)));
+    prev = __fsub_rn(prev, __fmul_rn(c.Bp, s));
+  }
+  last = xc;
+  h[2] = h[1];
+  h[1] = h[0];
+  h[0] = m;
+  return prev;
+}
+
+// Q = solver_order: the number of history buffers read and shifted.
+template <int Q>
+__global__ void unipc_step_kernel(const float* __restrict__ eps, const float* __restrict__ eps_text, float guidance,
+                                  const float* sample, const float* __restrict__ coef,
+                                  const int32_t* __restrict__ step_index, float* prev, float* __restrict__ last,
+                                  float* __restrict__ m1, float* __restrict__ m2, float* __restrict__ m3, long long n) {
+  const UniPCRow c = unipc_row(coef, step_index);
+  float* const hist[3] = {m1, m2, m3};
+  const long long nv = n / 4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+    const float4 e4 = __ldg(reinterpret_cast<const float4*>(eps) + i);
+    const float4 x4 = reinterpret_cast<const float4*>(sample)[i];
+    float ev[4] = {e4.x, e4.y, e4.z, e4.w};
+    if (eps_text) {
+      const float4 t = __ldg(reinterpret_cast<const float4*>(eps_text) + i);
+      const float tv[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) ev[j] = __fadd_rn(ev[j], __fmul_rn(guidance, __fsub_rn(tv[j], ev[j])));
+    }
+    const float xv[4] = {x4.x, x4.y, x4.z, x4.w};
+    float lv[4] = {0.f, 0.f, 0.f, 0.f};
+    if (c.q > 0) {
+      const float4 l = reinterpret_cast<const float4*>(last)[i];
+      lv[0] = l.x; lv[1] = l.y; lv[2] = l.z; lv[3] = l.w;
+    }
+    float hv[4][3] = {};
+#pragma unroll
+    for (int k = 0; k < Q; ++k) {
+      const float4 m = reinterpret_cast<const float4*>(hist[k])[i];
+      hv[0][k] = m.x; hv[1][k] = m.y; hv[2][k] = m.z; hv[3][k] = m.w;
+    }
+    float pv[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) pv[j] = unipc_elem(c, ev[j], xv[j], lv[j], hv[j]);
+    reinterpret_cast<float4*>(prev)[i] = make_float4(pv[0], pv[1], pv[2], pv[3]);
+    reinterpret_cast<float4*>(last)[i] = make_float4(lv[0], lv[1], lv[2], lv[3]);
+#pragma unroll
+    for (int k = 0; k < Q; ++k)
+      reinterpret_cast<float4*>(hist[k])[i] = make_float4(hv[0][k], hv[1][k], hv[2][k], hv[3][k]);
+  }
+  // tail
+  for (long long i = nv * 4 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+       i += (long long)gridDim.x * blockDim.x) {
+    float e = eps[i];
+    if (eps_text) e = __fadd_rn(e, __fmul_rn(guidance, __fsub_rn(eps_text[i], e)));
+    float l = c.q > 0 ? last[i] : 0.f;
+    float hv[3] = {};
+#pragma unroll
+    for (int k = 0; k < Q; ++k) hv[k] = hist[k][i];
+    prev[i] = unipc_elem(c, e, sample[i], l, hv);
+    last[i] = l;
+#pragma unroll
+    for (int k = 0; k < Q; ++k) hist[k][i] = hv[k];
   }
 }
 
@@ -364,6 +473,34 @@ extern "C" int ldm_dpmpp_step(const float* eps_uncond, const float* eps_text, fl
                                                                              x0_prev, n);
   count_launch();
   return check_launch("dpmpp_step_kernel");
+}
+
+extern "C" int ldm_unipc_step(const float* eps_uncond, const float* eps_text, float guidance_scale, const float* sample,
+                              const float* coef, const int32_t* step_index, float* prev_sample, float* last, float* m1,
+                              float* m2, float* m3, int32_t solver_order, int64_t n, ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(solver_order >= 1 && solver_order <= 3, LDM_ERR_BAD_ARG, "ldm_unipc_step: solver_order=%d",
+              (int)solver_order);
+  LDM_REQUIRE(eps_uncond && sample && coef && step_index && prev_sample && last && m1 && (solver_order < 2 || m2) &&
+                  (solver_order < 3 || m3),
+              LDM_ERR_BAD_ARG, "ldm_unipc_step: null arg");
+  LDM_REQUIRE(n > 0, LDM_ERR_BAD_SHAPE, "ldm_unipc_step: n=%lld", (long long)n);
+  LDM_REQUIRE(((uintptr_t)eps_uncond | (uintptr_t)eps_text | (uintptr_t)sample | (uintptr_t)prev_sample |
+               (uintptr_t)last | (uintptr_t)m1 | (uintptr_t)m2 | (uintptr_t)m3) % 16 == 0,
+              LDM_ERR_ALIGNMENT, "ldm_unipc_step: pointers must be 16-byte aligned");
+  const dim3 grid = grid_for(n / 4 + 1, 256);
+  auto s = as_stream(stream);
+  if (solver_order == 1)
+    unipc_step_kernel<1><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                              prev_sample, last, m1, m2, m3, n);
+  else if (solver_order == 2)
+    unipc_step_kernel<2><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                              prev_sample, last, m1, m2, m3, n);
+  else
+    unipc_step_kernel<3><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                              prev_sample, last, m1, m2, m3, n);
+  count_launch();
+  return check_launch("unipc_step_kernel");
 }
 
 extern "C" int ldm_timestep_sinusoid(const int64_t* timesteps, const int32_t* t_index, const float* freqs, float* out,

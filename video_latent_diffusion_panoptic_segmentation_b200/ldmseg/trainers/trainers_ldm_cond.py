@@ -4,7 +4,7 @@
 
 Data flow of one batch, all on the GPU:
   noise (CPU generator, as the reference) -> H2D
-  T x [ UNet CUDA graph (concat+cast fused into conv_in)  ->  fused DDIM (or DPM-Solver++) update ]      no host sync inside
+  T x [ UNet CUDA graph (concat+cast fused into conv_in)  ->  fused DDIM (DPM-Solver++, UniPC) update ]    no host sync inside
   seg-AE decoder (NHWC fp32 logits at 4h x 4w)
   fused bilinear x2 + argmax + softmax-max threshold + per-class areas  ->  merge filter  ->  int32 panoptic ids
   PQ / DVPQ statistics from joint id histograms
@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from ..evaluations.cityscapes_pap_eval import CityscapesPanopticEvaluator
-from ..schedulers import DPMSolverMultistepScheduler
+from ..schedulers import DPMSolverMultistepScheduler, UniPCMultistepScheduler
 from ..utils import color_map, get_world_size, is_dist_avail_and_initialized, is_main_process
 from ... import _lib as L
 from ... import ops
@@ -96,10 +96,11 @@ class TrainerDiffusion:
         return latents * scaling_factor, latents_mean * scaling_factor
 
     # ------------------------------------------------------------------ sample (:1048-1173)
-    def _loop_state(self, B, h, w, multiplier=1, ctx_len=None, dpm=False):
+    def _loop_state(self, B, h, w, multiplier=1, ctx_len=None, dpm=False, unipc_order=0):
         """Static buffers + UNet plan for the DDIM loop at this shape (built once, reused for every batch). With
         classifier-free guidance (multiplier 2) the UNet runs on the doubled batch [uncond | text] (:1129,1126).
-        dpm: also the x0_prev buffer of the DPM-Solver++ loop (same plan)."""
+        dpm: also the x0_prev buffer of the DPM-Solver++ loop (same plan). unipc_order: also the buffers of the UniPC
+        loop at that solver order, the corrected sample `unipc_last` and the x0 history `unipc_hist` (same plan)."""
         key = (B, h, w, self.self_condition, multiplier, ctx_len)
         st = self._loop.get(key)
         if st is None:
@@ -114,6 +115,11 @@ class TrainerDiffusion:
             self._loop[key] = st
         if dpm and "x0_prev" not in st:  # the DPM-Solver++ update's previous x0 prediction
             st["x0_prev"] = torch.empty((B, 4, h, w), dtype=f32, device=self.device)
+        if unipc_order:
+            if "unipc_last" not in st:
+                st["unipc_last"], st["unipc_hist"] = torch.empty((B, 4, h, w), dtype=f32, device=self.device), []
+            while len(st["unipc_hist"]) < unipc_order:
+                st["unipc_hist"].append(torch.empty((B, 4, h, w), dtype=f32, device=self.device))
         return st
 
     def norm_resize_images(self, x):
@@ -161,12 +167,17 @@ class TrainerDiffusion:
             scheduler = self.noise_scheduler
             scheduler.set_timesteps_inference(num_inference_steps)
         dpm = isinstance(scheduler, DPMSolverMultistepScheduler)
-        if not dpm and not (hasattr(scheduler, "coef_table") and hasattr(scheduler, "clip_range")):
+        unipc = isinstance(scheduler, UniPCMultistepScheduler)
+        if not (dpm or unipc) and not (hasattr(scheduler, "coef_table") and hasattr(scheduler, "clip_range")):
             raise NotImplementedError(f"sample: scheduler {type(scheduler).__name__} is not supported: pass this "
-                                      "package's DDIMNoiseScheduler or DPMSolverMultistepScheduler")
+                                      "package's DDIMNoiseScheduler, DPMSolverMultistepScheduler or "
+                                      "UniPCMultistepScheduler")
         if dpm and self.self_condition:
             raise NotImplementedError("self_condition with DPMSolverMultistepScheduler: the condition is the step's "
                                       "pred_original_sample (:1152-1153), which the DPM-Solver step output does not carry")
+        if unipc and self.self_condition:
+            raise NotImplementedError("self_condition with UniPCMultistepScheduler: the condition is the step's "
+                                      "pred_original_sample (:1152-1153), which the UniPC step output does not carry")
         if rgb_latents is None:
             raise NotImplementedError("unconditional sampling (rgb_latents=None) is not on the eval path")
         if repeat_noise is None:
@@ -188,7 +199,8 @@ class TrainerDiffusion:
             raise NotImplementedError("self_condition with a text encoder: the reference concatenates a doubled batch "
                                       "with an undoubled condition (:1134-1136,1152-1153) and fails")
         B = batch_size
-        st = self._loop_state(B, h, w, multiplier, ctx_len=None if ctx is None else ctx.shape[1], dpm=dpm)
+        st = self._loop_state(B, h, w, multiplier, ctx_len=None if ctx is None else ctx.shape[1], dpm=dpm,
+                              unipc_order=scheduler.solver_order if unipc else 0)
         lat_all, plan = st["latents"], st["plan"]
         latents = lat_all[:B]
         latents.copy_(noise.to(dev, non_blocking=True))           # H2D (:1095)
@@ -206,6 +218,9 @@ class TrainerDiffusion:
         if dpm:
             return self._dpm_loop(st, latents, B, multiplier, scheduler, timesteps, guidance_scale, return_all_latents,
                                   original_noise)
+        if unipc:
+            return self._unipc_loop(st, latents, B, multiplier, scheduler, timesteps, guidance_scale,
+                                    return_all_latents, original_noise)
         coef = scheduler.coef_table(dev)
         clip = scheduler.clip_range()  # scheduler.step's clip_sample (:1152-1154 calls it with its defaults)
         all_latents = []
@@ -255,6 +270,34 @@ class TrainerDiffusion:
             else:
                 self.unet_model._run_plan(plan)
             ops.dpmpp_step(plan.out[:B], latents, coef, steps[i:i + 1], prev_sample=latents, x0_prev=x0_prev,
+                           eps_text=plan.out[B:] if multiplier > 1 else None, guidance_scale=guidance_scale)
+            if return_all_latents:
+                all_latents.append(latents.clone())
+        if return_all_latents:
+            return torch.cat(all_latents, dim=0)
+        out = latents.clone()
+        if original_noise is not None:
+            return out, original_noise
+        return out
+
+    def _unipc_loop(self, st, latents, B, multiplier, scheduler, timesteps, guidance_scale, return_all_latents,
+                    original_noise):
+        """The sampler loop of sample() with a UniPCMultistepScheduler: the same UNet graph, then one fused UniPC
+        update (guidance, corrector of the previous step, predictor, history shift) per step. Its last step goes to
+        sigma = 0, where prev equals the final x0 prediction, as DDIM's last step leaves the latents."""
+        dev, lat_all, plan = self.device, st["latents"], st["plan"]
+        coef, steps = scheduler.coef_table(dev), scheduler.step_index_table(dev)
+        last, hist = st["unipc_last"], st["unipc_hist"][:scheduler.solver_order]
+        all_latents = []
+        for i in range(timesteps.numel()):
+            plan.timestep.copy_(timesteps[i:i + 1])
+            if multiplier > 1:
+                lat_all[B:].copy_(latents)
+            if plan.graph is not None:
+                plan.graph.replay()
+            else:
+                self.unet_model._run_plan(plan)
+            ops.unipc_step(plan.out[:B], latents, coef, steps[i:i + 1], prev_sample=latents, last=last, history=hist,
                            eps_text=plan.out[B:] if multiplier > 1 else None, guidance_scale=guidance_scale)
             if return_all_latents:
                 all_latents.append(latents.clone())

@@ -309,6 +309,36 @@ def dpmpp_step(eps, sample, coef, step_index, prev_sample, x0_prev, eps_text=Non
                                    _p(prev_sample), _p(x0_prev), n, _stream()), "ldm_dpmpp_step")
 
 
+def unipc_step(eps, sample, coef, step_index, prev_sample, last, history, eps_text=None, guidance_scale=0.0):
+    """UniPC update with the scalars of row *step_index of coef (f32 [steps, 20], UniPCMultistepScheduler): corrects
+    the previous step's result with `last` (the sample that step started from, corrected), then predicts prev_sample.
+    history = [m1, .., m_order], the previous x0 predictions, newest first; last and history are updated in place.
+    eps_text given: classifier-free guidance first, as ddim_step. prev_sample may be sample."""
+    history = list(history)
+    order = len(history)
+    if not 1 <= order <= 3:
+        raise L.LdmError(f"unipc_step: history holds the x0 predictions of solver orders 1 to 3, got {order}")
+    for t, nm in ((eps, "eps"), (sample, "sample"), (coef, "coef"), (prev_sample, "prev"), (last, "last"),
+                  (eps_text, "eps_text"), *((m, f"m{k + 1}") for k, m in enumerate(history))):
+        _chk(t, f32, nm)
+    _chk(step_index, i32, "step_index")
+    n = sample.numel()
+    for t, name in ((eps, "eps"), (prev_sample, "prev"), (last, "last"), (eps_text, "eps_text"),
+                    *((m, f"m{k + 1}") for k, m in enumerate(history))):
+        if t is not None and t.numel() != n:
+            raise L.LdmError(f"unipc_step: {name} has {t.numel()} elements, sample {n}")
+    owned = [last] + history
+    if len({t.data_ptr() for t in owned}) != len(owned) or any(
+            t.data_ptr() in (sample.data_ptr(), prev_sample.data_ptr()) for t in owned):
+        raise L.LdmError("unipc_step: last and the history buffers must not alias each other, sample or prev")
+    if coef.dim() != 2 or coef.shape[1] != 20 or step_index.numel() != 1:
+        raise L.LdmError("unipc_step: coef must be [steps, 20] and step_index one int32 element")
+    m = history + [None] * (3 - order)
+    L.check(L.lib().ldm_unipc_step(_p(eps), _p(eps_text), float(guidance_scale), _p(sample), _p(coef), _p(step_index),
+                                   _p(prev_sample), _p(last), _p(m[0]), _p(m[1]), _p(m[2]), order, n, _stream()),
+            "ldm_unipc_step")
+
+
 def upsample_nearest(x, out):
     _chk(x, bf16, "x"); _chk(out, bf16, "out")
     B, h, w, Cc = x.shape
