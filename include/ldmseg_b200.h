@@ -290,6 +290,31 @@ int ldm_unipc_step(const float* eps_uncond, const float* eps_text, float guidanc
                    const float* coef, const int32_t* step_index, float* prev_sample, float* last, float* m1, float* m2,
                    float* m3, int32_t solver_order, int64_t n, ldm_stream_t stream);
 
+/* Per-image timesteps (the streaming sampler: every image of a batch at its own step of its own trajectory). Each
+ * output element takes exactly the arithmetic of the single-timestep entry point above it, so image b's slice is bit
+ * for bit what that entry point gives for image b's timestep or row.
+ *   ldm_timestep_sinusoid_rows: out [B, 2*half], row b from t = timesteps[b] (int64 device [B]).
+ *   ldm_gemv_bf16_rows: x f32 [B, K] -> out[b][n] = act(bias[n] + bias2[n] + w[n,:] . x[b]), as ldm_gemv_bf16. With
+ *     seg_offs == NULL out is [B, N]; otherwise seg_offs is a device int32 [nseg + 1] of ascending column offsets from
+ *     0 to N, and out is segment-major: segment s (columns [o_s, o_{s+1})) is a contiguous [B, o_{s+1} - o_s] block at
+ *     float offset o_s * B -- the rowbias (ldm_gemm_desc.rowbias) of every resnet's conv1 from one launch.
+ *   ldm_ddim_step_rows / ldm_dpmpp_step_rows / ldm_unipc_step_rows: the updates of ldm_ddim_step / ldm_dpmpp_step /
+ *     ldm_unipc_step without guidance, element i reading coefficient row rows[i / elems_per_image] (device int32, one
+ *     entry per image; DDIM: the timestep value, as *t_index; DPM-Solver++ and UniPC: the step index).
+ *     elems_per_image is a positive multiple of 4; n need not be a multiple of it (the last image may be partial). */
+int ldm_timestep_sinusoid_rows(const int64_t* timesteps, const float* freqs, float* out, int32_t half, int32_t B,
+                               ldm_stream_t stream);
+int ldm_gemv_bf16_rows(const void* w, const float* bias, const float* bias2, const float* x, float* out, int32_t N,
+                       int32_t K, int32_t B, const int32_t* seg_offs, int32_t nseg, int32_t silu_out,
+                       ldm_stream_t stream);
+int ldm_ddim_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                       float* prev_sample, float* pred_x0, int64_t n, int64_t elems_per_image, ldm_stream_t stream);
+int ldm_dpmpp_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                        float* prev_sample, float* x0_prev, int64_t n, int64_t elems_per_image, ldm_stream_t stream);
+int ldm_unipc_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                        float* prev_sample, float* last, float* m1, float* m2, float* m3, int32_t solver_order,
+                        int64_t n, int64_t elems_per_image, ldm_stream_t stream);
+
 /* Layout helpers (NHWC bf16). */
 int ldm_upsample_nearest(const void* x, void* out, int32_t B, int32_t h, int32_t w, int32_t C, int32_t oh,
                          int32_t ow, ldm_stream_t stream); /* F.interpolate(mode="nearest") */

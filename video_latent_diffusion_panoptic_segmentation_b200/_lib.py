@@ -84,6 +84,11 @@ SIGNATURES = {
     "ldm_dpmpp_step": (C.c_int, [c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "ldm_unipc_step": (C.c_int, [c_vp, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i64,
                                  c_vp]),
+    "ldm_timestep_sinusoid_rows": (C.c_int, [c_vp, c_vp, c_vp, c_i32, c_i32, c_vp]),
+    "ldm_gemv_bf16_rows": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_vp]),
+    "ldm_ddim_step_rows": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp]),
+    "ldm_dpmpp_step_rows": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp]),
+    "ldm_unipc_step_rows": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i64, c_i64, c_vp]),
     "ldm_upsample_nearest": (C.c_int, [c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp]),
     "ldm_im2col3x3_s2": (C.c_int, [c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp]),
     "ldm_logits_to_ids": (C.c_int, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_f32, c_i32, c_vp]),

@@ -13,19 +13,35 @@ using namespace ldm;
 // `prev` / `x0out` may alias `sample` (in-place update by the sampler loop): no __restrict__ on those.
 // With `eps_text` the noise prediction is first combined as classifier-free guidance does (trainers_ldm_cond.py:1147-1149):
 // eps = eps_uncond + g * (eps_text - eps_uncond), three roundings in the reference's order.
+// kRows: t_index holds one row per image, element i reads row t_index[i / epi] (epi % 4 == 0, so a float4 lies in one
+// image); the row's scalars are reloaded only when a thread's element moves to another image.
+template <bool kRows>
 __global__ void ddim_step_kernel(const float* __restrict__ eps, const float* __restrict__ eps_text, float guidance,
                                  const float* sample, const float* __restrict__ coef,
                                  const int32_t* __restrict__ t_index, float* prev, float* x0out, long long n,
-                                 float clip, int reclip_eps) {
+                                 float clip, int reclip_eps, long long epi) {
   // clip > 0: pred_original_sample is clamped to [-clip, clip] (clip_sample, :253-257); reclip_eps: the noise is then
   // re-derived from the clamped x0 (use_clipped_model_output, :259-261), both in the reference's op order
-  const int ti = t_index ? *t_index : 0;
-  const float s1m_at = coef[ti * 4 + 0];   // sqrt(1 - alpha_t)
-  const float s_at = coef[ti * 4 + 1];     // sqrt(alpha_t)
-  const float s_ap = coef[ti * 4 + 2];     // sqrt(alpha_prev)
-  const float s1m_ap = coef[ti * 4 + 3];   // sqrt(1 - alpha_prev)
+  const int ti = kRows ? 0 : (t_index ? *t_index : 0);
+  float s1m_at = coef[ti * 4 + 0];   // sqrt(1 - alpha_t)
+  float s_at = coef[ti * 4 + 1];     // sqrt(alpha_t)
+  float s_ap = coef[ti * 4 + 2];     // sqrt(alpha_prev)
+  float s1m_ap = coef[ti * 4 + 3];   // sqrt(1 - alpha_prev)
+  long long img = 0;
+  auto select = [&](long long elem) {
+    if constexpr (kRows) {
+      if (elem / epi != img) {
+        img = elem / epi;
+        const int r = __ldg(t_index + img);
+        s1m_at = __ldg(coef + r * 4 + 0); s_at = __ldg(coef + r * 4 + 1);
+        s_ap = __ldg(coef + r * 4 + 2); s1m_ap = __ldg(coef + r * 4 + 3);
+      }
+    }
+  };
+  if constexpr (kRows) img = -1;
   const long long nv = n / 4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+    select(i * 4);
     const float4 e = __ldg(reinterpret_cast<const float4*>(eps) + i);
     const float4 x = reinterpret_cast<const float4*>(sample)[i];
     float ev[4] = {e.x, e.y, e.z, e.w};
@@ -50,6 +66,7 @@ __global__ void ddim_step_kernel(const float* __restrict__ eps, const float* __r
   // tail
   for (long long i = nv * 4 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
+    select(i);
     float e = eps[i];
     if (eps_text) e = __fadd_rn(e, __fmul_rn(guidance, __fsub_rn(eps_text[i], e)));
     float p0 = __fdiv_rn(__fsub_rn(sample[i], __fmul_rn(s1m_at, e)), s_at);
@@ -64,17 +81,35 @@ __global__ void ddim_step_kernel(const float* __restrict__ eps, const float* __r
 // Row *step_index of `coef` (ldmseg/schedulers/dpm_solver.py) holds {sig_i, alpha_i, A, Bc, c, hb, order, 0}:
 //   x0 = (x - sig_i * eps) / alpha_i;  prev = A * x - Bc * x0  [ - hb * (c * (x0 - x0_prev)) when order == 2 ]
 // in that op order with round-to-nearest intrinsics, as ddim_step_kernel. x0 replaces x0_prev in place (the same thread
-// reads and writes each element); `prev` may alias `sample`.
+// reads and writes each element); `prev` may alias `sample`. kRows: row step_index[i / epi] per image, as
+// ddim_step_kernel<true>.
 constexpr int kDpmCoefCols = 8;
+template <bool kRows>
 __global__ void dpmpp_step_kernel(const float* __restrict__ eps, const float* __restrict__ eps_text, float guidance,
                                   const float* sample, const float* __restrict__ coef,
-                                  const int32_t* __restrict__ step_index, float* prev, float* x0_prev, long long n) {
-  const float* row = coef + (long long)__ldg(step_index) * kDpmCoefCols;
-  const float sig = __ldg(row + 0), alpha = __ldg(row + 1), A = __ldg(row + 2), Bc = __ldg(row + 3);
-  const float c = __ldg(row + 4), hb = __ldg(row + 5);
-  const bool second = __ldg(row + 6) > 1.5f;
+                                  const int32_t* __restrict__ step_index, float* prev, float* x0_prev, long long n,
+                                  long long epi) {
+  float sig, alpha, A, Bc, c, hb;
+  bool second;
+  auto load = [&](const int32_t* idx) {
+    const float* row = coef + (long long)__ldg(idx) * kDpmCoefCols;
+    sig = __ldg(row + 0); alpha = __ldg(row + 1); A = __ldg(row + 2); Bc = __ldg(row + 3);
+    c = __ldg(row + 4); hb = __ldg(row + 5);
+    second = __ldg(row + 6) > 1.5f;
+  };
+  long long img = -1;
+  auto select = [&](long long elem) {
+    if constexpr (kRows) {
+      if (elem / epi != img) {
+        img = elem / epi;
+        load(step_index + img);
+      }
+    }
+  };
+  if constexpr (!kRows) load(step_index);
   const long long nv = n / 4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+    select(i * 4);
     const float4 e = __ldg(reinterpret_cast<const float4*>(eps) + i);
     const float4 x = reinterpret_cast<const float4*>(sample)[i];
     float ev[4] = {e.x, e.y, e.z, e.w};
@@ -103,6 +138,7 @@ __global__ void dpmpp_step_kernel(const float* __restrict__ eps, const float* __
   // tail
   for (long long i = nv * 4 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
+    select(i);
     float e = eps[i];
     if (eps_text) e = __fadd_rn(e, __fmul_rn(guidance, __fsub_rn(eps_text[i], e)));
     const float x = sample[i];
@@ -166,16 +202,29 @@ __device__ __forceinline__ float unipc_elem(const UniPCRow& c, float e, float x,
   return prev;
 }
 
-// Q = solver_order: the number of history buffers read and shifted.
-template <int Q>
+// Q = solver_order: the number of history buffers read and shifted. kRows: row step_index[i / epi] per image, as
+// ddim_step_kernel<true>.
+template <int Q, bool kRows>
 __global__ void unipc_step_kernel(const float* __restrict__ eps, const float* __restrict__ eps_text, float guidance,
                                   const float* sample, const float* __restrict__ coef,
                                   const int32_t* __restrict__ step_index, float* prev, float* __restrict__ last,
-                                  float* __restrict__ m1, float* __restrict__ m2, float* __restrict__ m3, long long n) {
-  const UniPCRow c = unipc_row(coef, step_index);
+                                  float* __restrict__ m1, float* __restrict__ m2, float* __restrict__ m3, long long n,
+                                  long long epi) {
+  UniPCRow c;
+  if constexpr (!kRows) c = unipc_row(coef, step_index);
+  long long img = -1;
+  auto select = [&](long long elem) {
+    if constexpr (kRows) {
+      if (elem / epi != img) {
+        img = elem / epi;
+        c = unipc_row(coef, step_index + img);
+      }
+    }
+  };
   float* const hist[3] = {m1, m2, m3};
   const long long nv = n / 4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
+    select(i * 4);
     const float4 e4 = __ldg(reinterpret_cast<const float4*>(eps) + i);
     const float4 x4 = reinterpret_cast<const float4*>(sample)[i];
     float ev[4] = {e4.x, e4.y, e4.z, e4.w};
@@ -209,6 +258,7 @@ __global__ void unipc_step_kernel(const float* __restrict__ eps, const float* __
   // tail
   for (long long i = nv * 4 + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
+    select(i);
     float e = eps[i];
     if (eps_text) e = __fadd_rn(e, __fmul_rn(guidance, __fsub_rn(eps_text[i], e)));
     float l = c.q > 0 ? last[i] : 0.f;
@@ -224,9 +274,12 @@ __global__ void unipc_step_kernel(const float* __restrict__ eps, const float* __
 
 // ---------------------------------------------------------------- timestep sinusoid (diffusers Timesteps)
 // out[0:half] = cos(t * f_i), out[half:2*half] = sin(t * f_i)   (flip_sin_to_cos=True, freq_shift=0)
+// kRows: one CTA per image b, t = timesteps[b], out row b of [B, 2*half].
+template <bool kRows>
 __global__ void timestep_sinusoid_kernel(const long long* __restrict__ timesteps, const int32_t* __restrict__ t_index,
                                          const float* __restrict__ freqs, float* __restrict__ out, int half) {
-  const float t = (float)timesteps[t_index ? *t_index : 0];
+  const float t = (float)timesteps[kRows ? (int)blockIdx.x : (t_index ? *t_index : 0)];
+  if constexpr (kRows) out += (long long)blockIdx.x * 2 * half;
   for (int i = threadIdx.x; i < half; i += blockDim.x) {
     const float a = __fmul_rn(t, freqs[i]);
     out[i] = cosf(a);
@@ -236,10 +289,15 @@ __global__ void timestep_sinusoid_kernel(const long long* __restrict__ timesteps
 
 // ---------------------------------------------------------------- GEMV: out[n] = act(bias[n] + bias2[n] + w[n,:] . x)
 // one warp per output row; x (fp32) staged in shared memory; w bf16 row-major [N,K], K % 8 == 0.
+// kRows: x is [B, K] with image b = blockIdx.y; out is [B, N], or with seg_offs (nseg + 1 ascending column offsets
+// from 0 to N) segment-major: column n of segment s lands at seg_offs[s] * B + b * width_s + (n - seg_offs[s]).
+// Every output element takes the arithmetic of the single-vector kernel, so row b equals it bit for bit.
+template <bool kRows>
 __global__ void gemv_bf16_kernel(const __nv_bfloat16* __restrict__ w, const float* __restrict__ bias,
                                  const float* __restrict__ bias2, const float* __restrict__ x, float* __restrict__ out,
-                                 int N, int K, int silu_out) {
+                                 int N, int K, int silu_out, const int32_t* __restrict__ seg_offs, int nseg) {
   extern __shared__ float xs[];
+  if constexpr (kRows) x += (long long)blockIdx.y * K;
   for (int i = threadIdx.x; i < K; i += blockDim.x) xs[i] = x[i];
   __syncthreads();
   const int lane = threadIdx.x & 31;
@@ -256,7 +314,19 @@ __global__ void gemv_bf16_kernel(const __nv_bfloat16* __restrict__ w, const floa
     acc = warp_sum(acc);
     if (lane == 0) {
       float v = acc + (bias ? bias[n] : 0.f) + (bias2 ? bias2[n] : 0.f);
-      out[n] = silu_out ? silu_f(v) : v;
+      long long o = n;
+      if constexpr (kRows) {
+        const long long b = blockIdx.y, B = gridDim.y;
+        if (seg_offs) {
+          int s = 0;
+          while (s + 1 < nseg && n >= seg_offs[s + 1]) ++s;
+          const int lo = seg_offs[s];
+          o = lo * B + b * (seg_offs[s + 1] - lo) + (n - lo);
+        } else {
+          o = b * N + n;
+        }
+      }
+      out[o] = silu_out ? silu_f(v) : v;
     }
   }
 }
@@ -450,10 +520,9 @@ extern "C" int ldm_ddim_step_clip(const float* eps_uncond, const float* eps_text
   LDM_REQUIRE(((uintptr_t)eps_uncond | (uintptr_t)eps_text | (uintptr_t)sample | (uintptr_t)prev_sample |
                (uintptr_t)pred_x0) % 16 == 0,
               LDM_ERR_ALIGNMENT, "ldm_ddim_step: pointers must be 16-byte aligned");
-  ddim_step_kernel<<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(eps_uncond, eps_text, guidance_scale, sample,
-                                                                            coef, t_index, prev_sample, pred_x0, n,
-                                                                            clip_sample_range,
-                                                                            use_clipped_model_output != 0);
+  ddim_step_kernel<false><<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(
+      eps_uncond, eps_text, guidance_scale, sample, coef, t_index, prev_sample, pred_x0, n, clip_sample_range,
+      use_clipped_model_output != 0, n);
   count_launch();
   return check_launch("ddim_step_kernel");
 }
@@ -468,9 +537,8 @@ extern "C" int ldm_dpmpp_step(const float* eps_uncond, const float* eps_text, fl
   LDM_REQUIRE(((uintptr_t)eps_uncond | (uintptr_t)eps_text | (uintptr_t)sample | (uintptr_t)prev_sample |
                (uintptr_t)x0_prev) % 16 == 0,
               LDM_ERR_ALIGNMENT, "ldm_dpmpp_step: pointers must be 16-byte aligned");
-  dpmpp_step_kernel<<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(eps_uncond, eps_text, guidance_scale,
-                                                                             sample, coef, step_index, prev_sample,
-                                                                             x0_prev, n);
+  dpmpp_step_kernel<false><<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(
+      eps_uncond, eps_text, guidance_scale, sample, coef, step_index, prev_sample, x0_prev, n, n);
   count_launch();
   return check_launch("dpmpp_step_kernel");
 }
@@ -491,14 +559,14 @@ extern "C" int ldm_unipc_step(const float* eps_uncond, const float* eps_text, fl
   const dim3 grid = grid_for(n / 4 + 1, 256);
   auto s = as_stream(stream);
   if (solver_order == 1)
-    unipc_step_kernel<1><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
-                                              prev_sample, last, m1, m2, m3, n);
+    unipc_step_kernel<1, false><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                                     prev_sample, last, m1, m2, m3, n, n);
   else if (solver_order == 2)
-    unipc_step_kernel<2><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
-                                              prev_sample, last, m1, m2, m3, n);
+    unipc_step_kernel<2, false><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                                     prev_sample, last, m1, m2, m3, n, n);
   else
-    unipc_step_kernel<3><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
-                                              prev_sample, last, m1, m2, m3, n);
+    unipc_step_kernel<3, false><<<grid, 256, 0, s>>>(eps_uncond, eps_text, guidance_scale, sample, coef, step_index,
+                                                     prev_sample, last, m1, m2, m3, n, n);
   count_launch();
   return check_launch("unipc_step_kernel");
 }
@@ -507,8 +575,8 @@ extern "C" int ldm_timestep_sinusoid(const int64_t* timesteps, const int32_t* t_
                                      int32_t half, ldm_stream_t stream) {
   using namespace ldm_host;
   LDM_REQUIRE(timesteps && freqs && out && half > 0, LDM_ERR_BAD_ARG, "ldm_timestep_sinusoid: bad arg");
-  timestep_sinusoid_kernel<<<1, 256, 0, as_stream(stream)>>>(reinterpret_cast<const long long*>(timesteps), t_index,
-                                                             freqs, out, half);
+  timestep_sinusoid_kernel<false><<<1, 256, 0, as_stream(stream)>>>(reinterpret_cast<const long long*>(timesteps),
+                                                                    t_index, freqs, out, half);
   count_launch();
   return check_launch("timestep_sinusoid_kernel");
 }
@@ -522,10 +590,104 @@ extern "C" int ldm_gemv_bf16(const void* w, const float* bias, const float* bias
   int grid = (N + wpb - 1) / wpb;
   const int cap = num_sms() * 8;
   if (grid > cap) grid = cap;
-  gemv_bf16_kernel<<<grid, wpb * 32, sizeof(float) * K, as_stream(stream)>>>(
-      reinterpret_cast<const __nv_bfloat16*>(w), bias, bias2, x, out, N, K, silu_out);
+  gemv_bf16_kernel<false><<<grid, wpb * 32, sizeof(float) * K, as_stream(stream)>>>(
+      reinterpret_cast<const __nv_bfloat16*>(w), bias, bias2, x, out, N, K, silu_out, nullptr, 0);
   count_launch();
   return check_launch("gemv_bf16_kernel");
+}
+
+// ---------------------------------------------------------------- per-image rows (streaming sampler)
+extern "C" int ldm_timestep_sinusoid_rows(const int64_t* timesteps, const float* freqs, float* out, int32_t half,
+                                          int32_t B, ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(timesteps && freqs && out && half > 0 && B > 0 && B <= 65535, LDM_ERR_BAD_ARG,
+              "ldm_timestep_sinusoid_rows: bad arg (half=%d, B=%d)", (int)half, (int)B);
+  timestep_sinusoid_kernel<true><<<B, 256, 0, as_stream(stream)>>>(reinterpret_cast<const long long*>(timesteps),
+                                                                   nullptr, freqs, out, half);
+  count_launch();
+  return check_launch("timestep_sinusoid_kernel");
+}
+
+extern "C" int ldm_gemv_bf16_rows(const void* w, const float* bias, const float* bias2, const float* x, float* out,
+                                  int32_t N, int32_t K, int32_t B, const int32_t* seg_offs, int32_t nseg,
+                                  int32_t silu_out, ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(w && x && out, LDM_ERR_BAD_ARG, "ldm_gemv_bf16_rows: null arg");
+  LDM_REQUIRE(N > 0 && K > 0 && K % 8 == 0 && K <= 8192 && B > 0 && B <= 65535, LDM_ERR_BAD_SHAPE,
+              "ldm_gemv_bf16_rows: N=%d K=%d B=%d", N, K, B);
+  LDM_REQUIRE(!seg_offs || nseg > 0, LDM_ERR_BAD_ARG, "ldm_gemv_bf16_rows: nseg=%d", nseg);
+  const int wpb = 8;
+  int grid = (N + wpb - 1) / wpb;
+  const int cap = num_sms() * 8;
+  if (grid > cap) grid = cap;
+  gemv_bf16_kernel<true><<<dim3(grid, B), wpb * 32, sizeof(float) * K, as_stream(stream)>>>(
+      reinterpret_cast<const __nv_bfloat16*>(w), bias, bias2, x, out, N, K, silu_out, seg_offs, nseg);
+  count_launch();
+  return check_launch("gemv_bf16_kernel");
+}
+
+static int check_rows_args(const char* what, const float* const* ptrs, int nptrs, const int32_t* rows, int64_t n,
+                           int64_t elems_per_image) {
+  using namespace ldm_host;
+  LDM_REQUIRE(rows != nullptr, LDM_ERR_BAD_ARG, "%s: null rows", what);
+  LDM_REQUIRE(n > 0 && elems_per_image > 0 && elems_per_image % 4 == 0, LDM_ERR_BAD_SHAPE,
+              "%s: n=%lld elems_per_image=%lld (a positive multiple of 4)", what, (long long)n,
+              (long long)elems_per_image);
+  uintptr_t a = 0;
+  for (int i = 0; i < nptrs; ++i) a |= (uintptr_t)ptrs[i];
+  LDM_REQUIRE(a % 16 == 0, LDM_ERR_ALIGNMENT, "%s: pointers must be 16-byte aligned", what);
+  return LDM_OK;
+}
+
+extern "C" int ldm_ddim_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                                  float* prev_sample, float* pred_x0, int64_t n, int64_t elems_per_image,
+                                  ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(eps && sample && coef, LDM_ERR_BAD_ARG, "ldm_ddim_step_rows: null arg");
+  const float* ptrs[] = {eps, sample, prev_sample, pred_x0};
+  if (int rc = check_rows_args("ldm_ddim_step_rows", ptrs, 4, rows, n, elems_per_image)) return rc;
+  ddim_step_kernel<true><<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(
+      eps, nullptr, 0.f, sample, coef, rows, prev_sample, pred_x0, n, 0.f, 0, elems_per_image);
+  count_launch();
+  return check_launch("ddim_step_kernel");
+}
+
+extern "C" int ldm_dpmpp_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                                   float* prev_sample, float* x0_prev, int64_t n, int64_t elems_per_image,
+                                   ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(eps && sample && coef && prev_sample && x0_prev, LDM_ERR_BAD_ARG, "ldm_dpmpp_step_rows: null arg");
+  const float* ptrs[] = {eps, sample, prev_sample, x0_prev};
+  if (int rc = check_rows_args("ldm_dpmpp_step_rows", ptrs, 4, rows, n, elems_per_image)) return rc;
+  dpmpp_step_kernel<true><<<grid_for(n / 4 + 1, 256), 256, 0, as_stream(stream)>>>(
+      eps, nullptr, 0.f, sample, coef, rows, prev_sample, x0_prev, n, elems_per_image);
+  count_launch();
+  return check_launch("dpmpp_step_kernel");
+}
+
+extern "C" int ldm_unipc_step_rows(const float* eps, const float* sample, const float* coef, const int32_t* rows,
+                                   float* prev_sample, float* last, float* m1, float* m2, float* m3,
+                                   int32_t solver_order, int64_t n, int64_t elems_per_image, ldm_stream_t stream) {
+  using namespace ldm_host;
+  LDM_REQUIRE(solver_order >= 1 && solver_order <= 3, LDM_ERR_BAD_ARG, "ldm_unipc_step_rows: solver_order=%d",
+              (int)solver_order);
+  LDM_REQUIRE(eps && sample && coef && prev_sample && last && m1 && (solver_order < 2 || m2) && (solver_order < 3 || m3),
+              LDM_ERR_BAD_ARG, "ldm_unipc_step_rows: null arg");
+  const float* ptrs[] = {eps, sample, prev_sample, last, m1, m2, m3};
+  if (int rc = check_rows_args("ldm_unipc_step_rows", ptrs, 7, rows, n, elems_per_image)) return rc;
+  const dim3 grid = grid_for(n / 4 + 1, 256);
+  auto s = as_stream(stream);
+  if (solver_order == 1)
+    unipc_step_kernel<1, true><<<grid, 256, 0, s>>>(eps, nullptr, 0.f, sample, coef, rows, prev_sample, last, m1, m2,
+                                                    m3, n, elems_per_image);
+  else if (solver_order == 2)
+    unipc_step_kernel<2, true><<<grid, 256, 0, s>>>(eps, nullptr, 0.f, sample, coef, rows, prev_sample, last, m1, m2,
+                                                    m3, n, elems_per_image);
+  else
+    unipc_step_kernel<3, true><<<grid, 256, 0, s>>>(eps, nullptr, 0.f, sample, coef, rows, prev_sample, last, m1, m2,
+                                                    m3, n, elems_per_image);
+  count_launch();
+  return check_launch("unipc_step_kernel");
 }
 
 extern "C" int ldm_conv3x3_small_cin(const float* s0, const float* s1, const float* s2, int32_t nsrc, int32_t cps,

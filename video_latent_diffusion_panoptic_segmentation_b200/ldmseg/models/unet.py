@@ -306,7 +306,7 @@ class UNet:
         self._packed = P
 
     # ------------------------------------------------------------------ plan
-    def _build_plan(self, B, h, w, cin, ctx_len=0):
+    def _build_plan(self, B, h, w, cin, ctx_len=0, per_image_t=False):
         if self._packed is None:
             self._pack()
         P, cfg, dev = self._packed, self.config, self.device
@@ -322,7 +322,11 @@ class UNet:
         st = SimpleNamespace()
         st.in_parts = None
         st.sample = torch.zeros((B, cin, h, w), dtype=f32, device=dev)     # static input (concatenated form)
-        st.timestep = torch.zeros((1,), dtype=torch.int64, device=dev)     # static timestep
+        st.per_image_t = per_image_t
+        if per_image_t:
+            st.timesteps = torch.zeros((B,), dtype=torch.int64, device=dev)  # static timestep of every image
+        else:
+            st.timestep = torch.zeros((1,), dtype=torch.int64, device=dev)   # static timestep
         st.out = torch.empty((B, cfg.out_channels, h, w), dtype=f32, device=dev)
         st.gn_stats = ops.gn_scratch(B, groups, dev)
         temb_dim = P["t1"][0].shape[0]
@@ -347,10 +351,25 @@ class UNet:
             plan.append((fn, a, k))
 
         # 1. time embedding chain (unet.py:301-307) -> per-resnet conv1 biases (conv1.bias + time_emb_proj(silu(emb)))
-        add(ops.timestep_sinusoid, st.timestep, None, P["freqs"], st.sinus)
-        add(ops.gemv, P["t1"][0], st.sinus, st.emb1, P["t1"][1], None, True)
-        add(ops.gemv, P["t2"][0], st.emb1, st.emb_silu, P["t2"][1], None, True)
-        add(ops.gemv, P["temb_w"], st.emb_silu, st.temb_bias, P["temb_b"], P["temb_conv1_b"], False)
+        if per_image_t:
+            # one embedding per image; the last GEMV writes segment-major [resnet][B][n_r], so every conv1 reads a
+            # contiguous [B, n_r] rowbias block. Each row's arithmetic is that of the single-vector chain.
+            st.sinus = torch.empty((B, 2 * P["freqs"].numel()), dtype=f32, device=dev)
+            st.emb1 = torch.empty((B, temb_dim), dtype=f32, device=dev)
+            st.emb_silu = torch.empty((B, temb_dim), dtype=f32, device=dev)
+            st.temb_rows = torch.empty((B * P["temb_total"],), dtype=f32, device=dev)
+            st.temb_seg_offs = torch.tensor(sorted(o for o, _ in P["temb_offs"].values()) + [P["temb_total"]],
+                                            dtype=torch.int32, device=dev)
+            add(ops.timestep_sinusoid_rows, st.timesteps, P["freqs"], st.sinus)
+            add(ops.gemv_rows, P["t1"][0], st.sinus, st.emb1, P["t1"][1], None, True)
+            add(ops.gemv_rows, P["t2"][0], st.emb1, st.emb_silu, P["t2"][1], None, True)
+            add(ops.gemv_rows, P["temb_w"], st.emb_silu, st.temb_rows, P["temb_b"], P["temb_conv1_b"], False,
+                seg_offs=st.temb_seg_offs)
+        else:
+            add(ops.timestep_sinusoid, st.timestep, None, P["freqs"], st.sinus)
+            add(ops.gemv, P["t1"][0], st.sinus, st.emb1, P["t1"][1], None, True)
+            add(ops.gemv, P["t2"][0], st.emb1, st.emb_silu, P["t2"][1], None, True)
+            add(ops.gemv, P["temb_w"], st.emb_silu, st.temb_bias, P["temb_b"], P["temb_conv1_b"], False)
 
         def resnet(name, xa, xb, H, W):
             c1 = xa.shape[-1]
@@ -360,7 +379,11 @@ class UNet:
             add(ops.groupnorm, xa, *P[name + ".norm1"], t0, st.gn_stats, x2=xb, groups=groups, eps=eps, silu=True)
             o, n = P["temb_offs"][name]
             t1 = arena.alloc((B, H, W, cout))
-            add(ops.gemm, t0, P[name + ".conv1"][0], t1, taps=9, bias=st.temb_bias[o:o + n])
+            if per_image_t:  # the epilogue adds 0 + rowbias: exactly the uniform plan's bias for that image's t
+                tb_ = dict(rowbias=st.temb_rows[o * B:(o + n) * B].view(B, n))
+            else:
+                tb_ = dict(bias=st.temb_bias[o:o + n])
+            add(ops.gemm, t0, P[name + ".conv1"][0], t1, taps=9, **tb_)
             arena.release(t0)
             t2 = arena.alloc((B, H, W, cout))
             add(ops.groupnorm, t1, *P[name + ".norm2"], t2, st.gn_stats, groups=groups, eps=eps, silu=True)
@@ -560,10 +583,12 @@ class UNet:
         st.context_in.view(B, st.ctx_len, -1).copy_(e)
         self._run_ctx_plan(st)
 
-    def _get_plan(self, B, h, w, cin, parts=None, ctx_len=None):
+    def _get_plan(self, B, h, w, cin, parts=None, ctx_len=None, per_image_t=False):
         """parts: optional list of static f32 NCHW [B,4,h,w] buffers (x_t, rgb_latents[, condition]) that conv_in
         reads directly -- the sampler's fused concat (trainers_ldm_cond.py:1134-1141). ctx_len: tokens of the
-        cross-attention context (default: the learnable object queries' count, or 0 without cross-attention)."""
+        cross-attention context (default: the learnable object queries' count, or 0 without cross-attention).
+        per_image_t: a plan whose static input is one timestep per image (`st.timesteps` int64 [B]) instead of one
+        for the batch (`st.timestep`); it has its own cache entry and CUDA graph."""
         if self._packed is None:
             self._pack()
         if ctx_len is None:
@@ -572,11 +597,13 @@ class UNet:
         if not self._packed["cross"]:
             ctx_len = 0
         key = (B, h, w, cin, ctx_len, None if parts is None else tuple(t.data_ptr() for t in parts))
+        if per_image_t:
+            key = key + ("per_image_t",)
         st = self._plans.get(key)
         if st is None:
             if cin != self.conv_in.in_channels:
                 raise ValueError(f"input has {cin} channels, conv_in expects {self.conv_in.in_channels}")
-            st = self._build_plan(B, h, w, cin, ctx_len)
+            st = self._build_plan(B, h, w, cin, ctx_len, per_image_t)
             if parts is not None:
                 self.set_split_inputs(st, parts)
             self._plans[key] = st
@@ -666,12 +693,18 @@ class UNet:
         use_ehs = cross and not learnable  # unet.py:322-323: learnable object queries replace whatever was passed
         if use_ehs and encoder_hidden_states is None:
             raise ValueError("this UNet keeps its cross-attention layers: encoder_hidden_states is required")
-        st = self._get_plan(B, h, w, cin, ctx_len=encoder_hidden_states.shape[1] if use_ehs else None)
+        ts = timestep if torch.is_tensor(timestep) else torch.tensor(timestep)
+        # diffusers' convention: a 1-D timestep of B elements gives every image its own timestep
+        per_image_t = ts.dim() == 1 and ts.numel() == B and B > 1
+        st = self._get_plan(B, h, w, cin, ctx_len=encoder_hidden_states.shape[1] if use_ehs else None,
+                            per_image_t=per_image_t)
         if use_ehs:
             self.set_context(st, encoder_hidden_states)
         st.sample.copy_(sample)
-        ts = timestep if torch.is_tensor(timestep) else torch.tensor(timestep)
-        st.timestep.copy_(ts.reshape(-1)[:1].to(torch.int64))  # unet.py:302-303: one timestep expanded over B
+        if per_image_t:
+            st.timesteps.copy_(ts.to(torch.int64))
+        else:
+            st.timestep.copy_(ts.reshape(-1)[:1].to(torch.int64))  # unet.py:302-303: one timestep expanded over B
         if st.graph is not None:
             st.graph.replay()
         else:

@@ -55,6 +55,7 @@ class TrainerDiffusion:
         self.device = torch.device("cuda", self.args["gpu"]) if isinstance(self.args["gpu"], int) else torch.device(
             self.args["gpu"])
         self._loop = {}
+        self._stream = {}
 
     # ------------------------------------------------------------------ encode_inputs (:336-396)
     @torch.no_grad()
@@ -308,6 +309,120 @@ class TrainerDiffusion:
             return out, original_noise
         return out
 
+    # ------------------------------------------------------------------ streaming sampler
+    def sample_stream(self, frames, num_inference_steps, scheduler=None, batch_size=8, seed=None):
+        """Sample a stream of frames through `batch_size` slots: every UNet forward advances each occupied slot by one
+        step of its own trajectory, a finished frame leaves its slot and the next frame takes it in the same forward.
+        That is the throughput of batch `batch_size` at a latency of N forwards per frame.
+
+        frames: iterable of (frame_id, rgb_latents [1,4,h,w], noise [1,4,h,w] or None); noise None is drawn from a CPU
+        generator seeded seed + frame_id (stream_noise). An item None means that no frame has arrived yet: the free
+        slots stay empty for that forward. Returns a generator of (frame_id, final latents [1,4,h,w]) in finishing
+        order. A frame's latents equal, bit for bit, those sample() gives it in a batch of `batch_size` at the same
+        position with the same noise. All frames take the same N; classifier-free guidance, self_condition, a
+        per-frame cross-attention context and DDIM's clip_sample are not built (learnable object queries are: their
+        context is the same for every frame)."""
+        if self.self_condition:
+            raise NotImplementedError("sample_stream: self_condition (the condition is each step's x0 prediction, "
+                                      "which the streaming updates do not carry)")
+        if self.textencoder is not None:
+            raise NotImplementedError("sample_stream: classifier-free guidance (a text encoder doubles the batch into "
+                                      "unconditional and conditional halves)")
+        if self.image_descriptor_model is not None and self.unet_model.has_cross_attention():
+            raise NotImplementedError("sample_stream: a cross-attention context that differs per frame (image "
+                                      "descriptors); learnable object queries are supported")
+        if scheduler is None:
+            scheduler = self.noise_scheduler
+            scheduler.set_timesteps_inference(num_inference_steps)
+        dpm = isinstance(scheduler, DPMSolverMultistepScheduler)
+        unipc = isinstance(scheduler, UniPCMultistepScheduler)
+        if not (dpm or unipc) and not (hasattr(scheduler, "coef_table") and hasattr(scheduler, "clip_range")):
+            raise NotImplementedError(f"sample_stream: scheduler {type(scheduler).__name__} is not supported: pass this "
+                                      "package's DDIMNoiseScheduler, DPMSolverMultistepScheduler or "
+                                      "UniPCMultistepScheduler")
+        if not (dpm or unipc) and scheduler.clip_range() != 0.0:
+            raise NotImplementedError("sample_stream: DDIM with clip_sample")
+        if batch_size < 1:
+            raise ValueError(f"sample_stream: batch_size={batch_size}")
+        return self._stream_loop(frames, scheduler, "dpm" if dpm else "unipc" if unipc else "ddim", batch_size, seed)
+
+    def _stream_state(self, B, h, w, kind, order):
+        """Static buffers of the streaming loop at this shape, and the UNet's per-image-timestep plan reading them."""
+        key = (B, h, w, kind, order)
+        st = self._stream.get(key)
+        if st is None:
+            dev = self.device
+            z = lambda: torch.zeros((B, 4, h, w), dtype=f32, device=dev)  # noqa: E731
+            st = {"latents": z(), "rgb": z(), "rows": torch.zeros((B,), dtype=i32, device=dev)}
+            st["plan"] = self.unet_model._get_plan(B, h, w, 8, parts=[st["latents"], st["rgb"]], per_image_t=True)
+            # host side of the per-forward copies, one set per forward in flight (see _stream_loop)
+            st["ts_host"] = torch.zeros((2, B), dtype=torch.int64).pin_memory()
+            st["rows_host"] = torch.zeros((2, B), dtype=i32).pin_memory()
+            st["noise_host"] = torch.zeros((2, B, 4, h, w), dtype=f32).pin_memory()
+            st["done"] = [torch.cuda.Event(), torch.cuda.Event()]
+            if kind == "ddim":
+                st["x0"] = z()             # the last step's result is its x0 prediction, as in sample()
+            elif kind == "dpm":
+                st["x0_prev"] = z()
+            else:
+                st["last"], st["hist"] = z(), [z() for _ in range(order)]
+            self._stream[key] = st
+        return st
+
+    @torch.no_grad()
+    def _stream_loop(self, frames, scheduler, kind, B, seed):
+        dev = self.device
+        timesteps = scheduler.timesteps.cpu().tolist()
+        N = len(timesteps)
+        coef = scheduler.coef_table(dev)
+        st, plan = None, None
+        for admitted, steps, finished in stream_schedule(frames, N, B):
+            if st is None:
+                h, w = admitted[0][1][1].shape[-2:]
+                st = self._stream_state(B, h, w, kind, scheduler.solver_order if kind == "unipc" else 0)
+                plan, lat, rgb, rows = st["plan"], st["latents"], st["rgb"], st["rows"]
+                fwd = 0
+            # The loop reads nothing back from the device: rows and timesteps go host -> device, a finished frame's
+            # latents are cloned on the device. Its one wait is on the forward before the previous one, which keeps the
+            # GPU one forward ahead of admission (a frame that arrives while a forward runs joins the next one) and
+            # frees that forward's set of pinned host buffers for reuse.
+            ring = fwd % 2
+            fwd += 1
+            st["done"][ring].synchronize()
+            ts_h, rows_h, noise_h = st["ts_host"][ring], st["rows_host"][ring], st["noise_host"][ring]
+            for s, (fid, rgb_f, noise) in admitted:
+                noise_h[s].copy_((noise if noise is not None else stream_noise(fid, seed, lat.shape[1:])).reshape(
+                    lat.shape[1:]))
+                lat[s].copy_(noise_h[s], non_blocking=True)
+                if scheduler.init_noise_sigma != 1.0:
+                    lat[s].mul_(scheduler.init_noise_sigma)
+                rgb[s].copy_(rgb_f.reshape(rgb.shape[1:]).to(dev, f32), non_blocking=True)
+            for s, i in enumerate(steps):
+                if i is None:               # an empty slot runs step 0 on zeros; its result is never read
+                    lat[s].zero_()
+                    rgb[s].zero_()
+                i = 0 if i is None else i
+                ts_h[s] = timesteps[i]
+                rows_h[s] = timesteps[i] if kind == "ddim" else i
+            plan.timesteps.copy_(ts_h, non_blocking=True)
+            rows.copy_(rows_h, non_blocking=True)
+            if plan.graph is not None:
+                plan.graph.replay()
+            else:
+                self.unet_model._run_plan(plan)
+            epi = lat[0].numel()
+            if kind == "ddim":
+                ops.ddim_step_rows(plan.out, lat, coef, rows, epi, prev_sample=lat, pred_x0=st["x0"])
+            elif kind == "dpm":
+                ops.dpmpp_step_rows(plan.out, lat, coef, rows, epi, prev_sample=lat, x0_prev=st["x0_prev"])
+            else:
+                ops.unipc_step_rows(plan.out, lat, coef, rows, epi, prev_sample=lat, last=st["last"],
+                                    history=st["hist"])
+            st["done"][ring].record()
+            final = st["x0"] if kind == "ddim" else lat   # DPM-Solver++ / UniPC end at sigma = 0, where prev is x0
+            for s, (fid, _, _) in finished:
+                yield fid, final[s:s + 1].clone()
+
     # ------------------------------------------------------------------ decode_latents (:398-444)
     @torch.no_grad()
     def decode_latents(self, latents, return_logits=False, threshold_output=False, rgb_latents=None,
@@ -490,6 +605,52 @@ class TrainerDiffusion:
         if is_dist_avail_and_initialized():
             torch.distributed.barrier()
         return self.last_results
+
+
+def stream_noise(frame_id, seed, shape):
+    """The initial noise of stream frame `frame_id` when it brings none: a CPU generator seeded seed + frame_id (the
+    default generator without a seed), shape [4, h, w]."""
+    gen = torch.Generator().manual_seed(seed + frame_id) if seed is not None else None
+    return torch.randn((1,) + tuple(shape), generator=gen)
+
+
+def stream_schedule(frames, num_steps, num_slots):
+    """Slot bookkeeping of TrainerDiffusion.sample_stream. Yields once per UNet forward (admitted, steps, finished):
+      admitted: [(slot, item)], the frames that enter a free slot at this forward, in arrival order (lowest free slot
+                first); a frame runs step 0 in the forward it enters;
+      steps:    per slot, the step it runs at this forward, or None for an empty slot;
+      finished: [(slot, item)], the frames whose last step this forward runs, in arrival order.
+    `frames` is pulled only while a slot is free. An item None means nothing has arrived yet: the remaining free slots
+    stay empty for this forward, and no forward is yielded while every slot is empty."""
+    it = iter(frames)
+    item, step = [None] * num_slots, [0] * num_slots
+    exhausted = False
+    while True:
+        admitted = []
+        for s in range(num_slots):
+            if exhausted or item[s] is not None:
+                continue
+            try:
+                nxt = next(it)
+            except StopIteration:
+                exhausted = True
+                continue
+            if nxt is None:
+                break
+            item[s], step[s] = nxt, 0
+            admitted.append((s, nxt))
+        if all(x is None for x in item):
+            if exhausted:
+                return
+            continue
+        # slots are filled lowest first, so within one forward slot order is arrival order
+        finished = [(s, item[s]) for s in range(num_slots) if item[s] is not None and step[s] == num_steps - 1]
+        yield admitted, [step[s] if item[s] is not None else None for s in range(num_slots)], finished
+        for s in range(num_slots):
+            if item[s] is not None:
+                step[s] += 1
+                if step[s] == num_steps:
+                    item[s] = None
 
 
 def p_get(p, key):

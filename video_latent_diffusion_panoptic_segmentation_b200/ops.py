@@ -251,6 +251,88 @@ def gemv(w, x, out, bias=None, bias2=None, silu=False):
     return out
 
 
+def timestep_sinusoid_rows(timesteps, freqs, out):
+    """timesteps int64 [B] -> out f32 [B, 2 * half]; row b equals timestep_sinusoid of timesteps[b] bit for bit."""
+    _chk(timesteps, i64, "timesteps"); _chk(freqs, f32, "freqs"); _chk(out, f32, "out")
+    B = timesteps.numel()
+    if out.numel() != B * 2 * freqs.numel():
+        raise L.LdmError(f"timestep_sinusoid_rows: out has {out.numel()} elements, expected {B} x {2 * freqs.numel()}")
+    L.check(L.lib().ldm_timestep_sinusoid_rows(_p(timesteps), _p(freqs), _p(out), freqs.numel(), B, _stream()),
+            "ldm_timestep_sinusoid_rows")
+    return out
+
+
+def gemv_rows(w, x, out, bias=None, bias2=None, silu=False, seg_offs=None):
+    """x f32 [B, K] -> out f32: row b equals gemv of x[b] bit for bit. out is [B, N], or with seg_offs (device int32
+    [nseg + 1], ascending column offsets from 0 to N) segment-major: segment s is a contiguous [B, width_s] block at
+    offset seg_offs[s] * B (ldm_gemv_bf16_rows)."""
+    _chk(w, bf16, "w"); _chk(x, f32, "x"); _chk(out, f32, "out"); _chk(bias, f32, "bias"); _chk(bias2, f32, "bias2")
+    _chk(seg_offs, i32, "seg_offs")
+    N, K = w.shape
+    B = x.numel() // K
+    if x.numel() != B * K or out.numel() != B * N:
+        raise L.LdmError(f"gemv_rows: x has {x.numel()} and out {out.numel()} elements for w [{N}, {K}]")
+    nseg = 0 if seg_offs is None else seg_offs.numel() - 1
+    L.check(L.lib().ldm_gemv_bf16_rows(_p(w), _p(bias), _p(bias2), _p(x), _p(out), N, K, B, _p(seg_offs), nseg,
+                                       int(silu), _stream()), "ldm_gemv_bf16_rows")
+    return out
+
+
+def _check_rows(what, sample, rows, elems_per_image, named):
+    """Shared checks of the *_step_rows wrappers: dtypes, element counts, one int32 row per (possibly partial) image."""
+    for t, nm in named:
+        _chk(t, f32, nm)
+    _chk(sample, f32, "sample"); _chk(rows, i32, "rows")
+    n = sample.numel()
+    for t, nm in named:
+        if nm != "coef" and t is not None and t.numel() != n:
+            raise L.LdmError(f"{what}: {nm} has {t.numel()} elements, sample {n}")
+    if elems_per_image <= 0 or elems_per_image % 4 or rows.numel() < -(-n // elems_per_image):
+        raise L.LdmError(f"{what}: elems_per_image={elems_per_image} (a positive multiple of 4) and one row per image "
+                         f"({rows.numel()} rows for {n} elements)")
+    return n
+
+
+def ddim_step_rows(eps, sample, coef, rows, elems_per_image, prev_sample=None, pred_x0=None):
+    """ddim_step without guidance or clipping, element i at coefficient row rows[i // elems_per_image] (the timestep
+    value, as t_index)."""
+    n = _check_rows("ddim_step_rows", sample, rows, elems_per_image,
+                    ((eps, "eps"), (coef, "coef"), (prev_sample, "prev"), (pred_x0, "x0")))
+    L.check(L.lib().ldm_ddim_step_rows(_p(eps), _p(sample), _p(coef), _p(rows), _p(prev_sample), _p(pred_x0), n,
+                                       elems_per_image, _stream()), "ldm_ddim_step_rows")
+
+
+def dpmpp_step_rows(eps, sample, coef, rows, elems_per_image, prev_sample, x0_prev):
+    """dpmpp_step without guidance, element i at row rows[i // elems_per_image] of coef (the step index)."""
+    n = _check_rows("dpmpp_step_rows", sample, rows, elems_per_image,
+                    ((eps, "eps"), (coef, "coef"), (prev_sample, "prev"), (x0_prev, "x0_prev")))
+    if coef.dim() != 2 or coef.shape[1] != 8:
+        raise L.LdmError("dpmpp_step_rows: coef must be [steps, 8]")
+    L.check(L.lib().ldm_dpmpp_step_rows(_p(eps), _p(sample), _p(coef), _p(rows), _p(prev_sample), _p(x0_prev), n,
+                                        elems_per_image, _stream()), "ldm_dpmpp_step_rows")
+
+
+def unipc_step_rows(eps, sample, coef, rows, elems_per_image, prev_sample, last, history):
+    """unipc_step without guidance, element i at row rows[i // elems_per_image] of coef (the step index)."""
+    history = list(history)
+    order = len(history)
+    if not 1 <= order <= 3:
+        raise L.LdmError(f"unipc_step_rows: history holds the x0 predictions of solver orders 1 to 3, got {order}")
+    n = _check_rows("unipc_step_rows", sample, rows, elems_per_image,
+                    ((eps, "eps"), (coef, "coef"), (prev_sample, "prev"), (last, "last"),
+                     *((m, f"m{k + 1}") for k, m in enumerate(history))))
+    owned = [last] + history
+    if len({t.data_ptr() for t in owned}) != len(owned) or any(
+            t.data_ptr() in (sample.data_ptr(), prev_sample.data_ptr()) for t in owned):
+        raise L.LdmError("unipc_step_rows: last and the history buffers must not alias each other, sample or prev")
+    if coef.dim() != 2 or coef.shape[1] != 20:
+        raise L.LdmError("unipc_step_rows: coef must be [steps, 20]")
+    m = history + [None] * (3 - order)
+    L.check(L.lib().ldm_unipc_step_rows(_p(eps), _p(sample), _p(coef), _p(rows), _p(prev_sample), _p(last), _p(m[0]),
+                                        _p(m[1]), _p(m[2]), order, n, elems_per_image, _stream()),
+            "ldm_unipc_step_rows")
+
+
 def pack_small_cin_weight(w):
     """Conv2d weight [cout, cin, 3, 3] (reference layout) -> f32 [cin, 3, 3, cout] for conv3x3_small_cin."""
     return w.detach().to(f32).permute(1, 2, 3, 0).contiguous()
